@@ -3,6 +3,7 @@
 
   python bench.py --gpus N --steps K --warmup W            (N>1: launched under torchrun, one rank/GPU)
   python bench.py --impl reference ...                     (the reference's CPU path, bounded sample)
+  python bench.py ... --dump-outputs DIR                   (also save a fixed sample of the last timed step's logits)
 
 A step = one prefill of the headline workload (configs[1]): batch 8, 336 px image, 8 RoIs per
 image, 128 text tokens -> L = 706, CLIP-ViT-L/14 + SPI module + LLaMA-7B + lm_head, bf16, random-init
@@ -346,7 +347,7 @@ def run_reference(args):
     if rank != 0:
         return
     t0 = time.perf_counter()
-    best = cpu_reference_sample(repeats=max(3, min(args.steps, 5)))
+    best = cpu_reference_sample(repeats=args.steps)
     L = WORKLOAD['text_tokens'] + (WORKLOAD['image_size'] // 14) ** 2 + 2
     line = dict(impl='reference', metric=METRIC, value=best['value'],
                 unit='samples/s', n_gpus=args.gpus, steps=len(best['repeat_seconds']), warmup=1,
@@ -487,6 +488,22 @@ def train_extra(dev, world, rank, steps=4, warmup=2, batch=4, stage1=True):
     return out
 
 
+DUMP_ROWS = 256   # sampled logit rows: 256 x 32006 fp32 = 33 MB
+
+
+def dump_logits(logits, out_dir):
+    """Write what the last timed step returned, the [B, L, V] logits, as float32 .npy files small enough to keep:
+    logits_last.npy = every sample's last position [B, V]; logits_rows.npy = DUMP_ROWS (b, l) positions drawn once
+    from a fixed seed, in ascending b * L + l order [DUMP_ROWS, V]."""
+    import numpy as np
+    B, L, V = logits.shape
+    rows = np.sort(np.random.default_rng(0).choice(B * L, size=min(DUMP_ROWS, B * L), replace=False))
+    flat = logits.reshape(B * L, V)
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, 'logits_last.npy'), logits[:, -1].float().cpu().numpy())
+    np.save(os.path.join(out_dir, 'logits_rows.npy'), flat[rows.tolist()].float().cpu().numpy())
+
+
 def run_ours(args):
     # keep stdout to the single JSON line: NCCL prints its version banner there unless told otherwise
     if os.environ.get('NCCL_DEBUG', 'VERSION').upper() == 'VERSION':
@@ -554,6 +571,8 @@ def run_ours(args):
     clocks = sampler.stop() if sampler else None
     ms_step = ms_total / args.steps
     value = world * B / (ms_step / 1e3)
+    if args.dump_outputs and rank == 0:
+        dump_logits(graph.out, args.dump_outputs)
 
     # ---- e2e: public API with pinned HOST buffers.  Every step: H2D of ids/images/boxes, graph replay, D2H of
     #      EVERYTHING the step computes (the full [B,L,V] logits, 361 MB) into pinned host memory.  The D2H runs on a
@@ -700,7 +719,11 @@ def main():
     ap.add_argument('--no-extras', action='store_true', help='headline only (no config2 / decode / train_step extras)')
     ap.add_argument('--no-train', action='store_true')
     ap.add_argument('--ncu', action='store_true', help='one eager forward inside a cudaProfiler window')
+    ap.add_argument('--dump-outputs', metavar='DIR',
+                    help='after the timed steps, write a fixed sample of the last step\'s logits to DIR/*.npy (float32)')
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error('--steps must be at least 1')
     if args.impl == 'reference':
         run_reference(args)
     else:

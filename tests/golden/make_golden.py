@@ -429,3 +429,88 @@ def input_pipeline_golden():
 
 if __name__ == '__main__' and '--input' in sys.argv:
     input_pipeline_golden()
+
+
+# ---------------------------------------------------------------------------------------------
+# Oracle pin on adversarial boxes: seeded maps and random + adversarial RoIs (tests/helpers.make_rois) through the
+# reference's CPU kernel compiled unmodified (oracle/_ref), avg with fixed and adaptive sampling and max pooling.
+# Stored: inputs, outputs and argmax -> tests/golden/roi_align_adversarial_ref.npz.
+# ---------------------------------------------------------------------------------------------
+ADVERSARIAL_CASES = [(48, 14, 2, 'avg', 7.0), (24, 7, 0, 'avg', 14.0), (16, 3, 2, 'max', 14.0)]   # H, PH, sr, mode, stride
+
+
+def adversarial_golden():
+    from tests.helpers import make_rois
+    ext = build_ref.load()
+    assert ext is not None, 'reference tree not available'
+    rng = np.random.default_rng(7)
+    store, meta = {}, []
+    for i, (H, PH, sr, mode, stride) in enumerate(ADVERSARIAL_CASES):
+        name = 'c%d' % i
+        x = rng.standard_normal((2, 5, H, H)).astype(np.float32)
+        rois = make_rois(rng, 2, 6, H * stride, adversarial=True)
+        scale = float(np.float32(1 / stride))
+        xt, rt = torch.from_numpy(x), torch.from_numpy(rois)
+        pm = 0 if mode == 'max' else 1
+        o = xt.new_zeros(len(rois), 5, PH, PH)
+        ay = xt.new_zeros(o.shape) if pm == 0 else xt.new_zeros(0)
+        ax = xt.new_zeros(o.shape) if pm == 0 else xt.new_zeros(0)
+        ext.roi_align_forward(xt, rt, o, ay, ax, aligned_height=PH, aligned_width=PH,
+                              spatial_scale=scale, sampling_ratio=sr, pool_mode=pm, aligned=True)
+        store[name + '.input'], store[name + '.rois'], store[name + '.output'] = x, rois, o.numpy()
+        if pm == 0:
+            store[name + '.argmax_y'], store[name + '.argmax_x'] = ay.numpy(), ax.numpy()
+        meta.append(dict(name=name, PH=PH, sampling_ratio=sr, pool_mode=mode, spatial_scale=scale))
+    store['meta'] = np.frombuffer(json.dumps(meta).encode(), dtype=np.uint8)
+    np.savez_compressed(os.path.join(HERE, 'roi_align_adversarial_ref.npz'), **store)
+    print('wrote roi_align_adversarial_ref.npz (%d cases)' % len(meta))
+
+
+if __name__ == '__main__' and '--adversarial' in sys.argv:
+    adversarial_golden()
+
+
+# ---------------------------------------------------------------------------------------------
+# How the reference's own wrapper (mmcv-1.4.7/mmcv/ops/roi_align.py, unmodified) calls `mmcv._ext`: every symbol that
+# `import mmcv.ops` asserts on (mmcv/utils/ext_loader.py), and the roi_align_forward / roi_align_backward calls of a
+# RoIAlign forward + backward in 'avg' and 'max' mode (tensor arguments by shape and dtype, scalars by value).
+# Recorded over the reference CPU kernel (oracle/_ref) -> tests/golden/mmcv_wrapper_calls.json.
+# ---------------------------------------------------------------------------------------------
+def wrapper_calls_golden():
+    sys.path.insert(0, HERE)
+    import importlib
+    import ref_shims
+    ref_shims.install()
+    ext_loader = importlib.import_module('mmcv.utils.ext_loader')
+    names = set()
+    load_ext = ext_loader.load_ext
+
+    def recording_load_ext(name, funcs):
+        if name == '_ext':
+            names.update(funcs)
+        return load_ext(name, funcs)
+    ext_loader.load_ext = recording_load_ext
+    importlib.import_module('mmcv.ops')
+    R = sys.modules['mmcv.ops.roi_align']
+
+    def describe(v):
+        if isinstance(v, torch.Tensor):
+            return dict(shape=list(v.shape), dtype=str(v.dtype).replace('torch.', ''))
+        return v
+    calls = []
+    for fn in ('roi_align_forward', 'roi_align_backward'):
+        def recorder(*args, _fn=fn, _impl=getattr(R.ext_module, fn), **kwargs):
+            calls.append(dict(fn=_fn, args=[describe(a) for a in args], kwargs={k: describe(v) for k, v in kwargs.items()}))
+            return _impl(*args, **kwargs)
+        setattr(R.ext_module, fn, recorder)
+    for mode in ('avg', 'max'):
+        x = torch.randn(1, 4, 8, 8, requires_grad=True)
+        R.RoIAlign((7, 7), 0.5, 2, mode)(x, torch.tensor([[0., 0., 0., 4., 4.]])).sum().backward()
+    doc = dict(source='mmcv-1.4.7/mmcv/ops/roi_align.py over mmcv/utils/ext_loader.py', ext_names=sorted(names), calls=calls)
+    with open(os.path.join(HERE, 'mmcv_wrapper_calls.json'), 'w') as f:
+        json.dump(doc, f, indent=1)
+    print('wrote mmcv_wrapper_calls.json (%d symbols, %d calls)' % (len(names), len(calls)))
+
+
+if __name__ == '__main__' and '--wrapper' in sys.argv:
+    wrapper_calls_golden()

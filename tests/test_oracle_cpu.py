@@ -1,12 +1,14 @@
 """CPU tests: pin the oracle (oracle/roi_align_oracle.c) against the reference's own
-known-answer vectors, the committed golden fixtures (outputs of the reference kernel
-compiled from its sources) and -- when oracle/_ref is present -- the live reference."""
+known-answer vectors and the committed golden fixtures (outputs of the reference kernel
+compiled from its sources)."""
+import json
+import os
+
 import numpy as np
 import pytest
 
-from oracle import build_ref
 from oracle import roi_align_oracle as O
-from tests.helpers import load_kat, load_ref_cases, make_rois
+from tests.helpers import GOLDEN, load_kat, load_ref_cases, make_rois
 
 
 @pytest.mark.parametrize('dtype', [np.float32, np.float64])
@@ -71,27 +73,19 @@ def test_oracle_empty_rois():
 
 
 def test_oracle_matches_live_reference_build():
-    """oracle/_ref = the reference's cpu/roi_align.cpp compiled unmodified (when available)."""
-    ext = build_ref.load()
-    if ext is None:
-        pytest.skip('oracle/_ref not built and /root/reference absent')
-    import torch
-    rng = np.random.default_rng(7)
-    for (H, PH, sr, mode, stride) in [(48, 14, 2, 'avg', 7.0), (24, 7, 0, 'avg', 14.0), (16, 3, 2, 'max', 14.0)]:
-        x = rng.standard_normal((2, 5, H, H)).astype(np.float32)
-        rois = make_rois(rng, 2, 6, H * stride, adversarial=True)
-        scale = float(np.float32(1 / stride))
-        out, ay, ax = O.roi_align_forward(x, rois, PH, scale, sr, mode, True)
-        xt, rt = torch.from_numpy(x), torch.from_numpy(rois)
-        o = xt.new_zeros(out.shape)
-        pm = 0 if mode == 'max' else 1
-        ayt = xt.new_zeros(out.shape) if pm == 0 else xt.new_zeros(0)
-        axt = xt.new_zeros(out.shape) if pm == 0 else xt.new_zeros(0)
-        ext.roi_align_forward(xt, rt, o, ayt, axt, aligned_height=PH, aligned_width=PH,
-                              spatial_scale=scale, sampling_ratio=sr, pool_mode=pm, aligned=True)
-        assert np.array_equal(out, o.numpy())
-        if pm == 0:
-            assert np.array_equal(ay, ayt.numpy()) and np.array_equal(ax, axt.numpy())
+    """The reference's cpu/roi_align.cpp compiled unmodified (oracle/_ref), run on seeded random + adversarial boxes
+    (tests/golden/roi_align_adversarial_ref.npz, written by make_golden.py --adversarial): the oracle reproduces its
+    outputs and argmax bit for bit."""
+    z = np.load(os.path.join(GOLDEN, 'roi_align_adversarial_ref.npz'))
+    meta = json.loads(bytes(z['meta']).decode())
+    assert len(meta) == 3
+    for m in meta:
+        n = m['name']
+        out, ay, ax = O.roi_align_forward(z[n + '.input'], z[n + '.rois'], m['PH'], m['spatial_scale'],
+                                          m['sampling_ratio'], m['pool_mode'], True)
+        assert np.array_equal(out, z[n + '.output']), n
+        if m['pool_mode'] == 'max':
+            assert np.array_equal(ay, z[n + '.argmax_y']) and np.array_equal(ax, z[n + '.argmax_x']), n
 
 
 # ---------------------------------------------------------------------------------------

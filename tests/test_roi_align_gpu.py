@@ -54,8 +54,8 @@ def test_mmcv_ext_module_as_the_reference_wrapper_calls_it():
     """The `mmcv._ext` drop-in module (gpt4roi_b200.mmcv_ext, what `install()` registers), called exactly the way the
     reference's own wrapper calls it -- mmcv-1.4.7/mmcv/ops/roi_align.py:83-96 (forward: `new_zeros` output / argmax
     buffers, five positional tensors, six keyword scalars) and :113-123 (backward) -- on the mmcv known-answer cases and on
-    a pyramid-sized fp32 case against the oracle (bit-exact forward).  tests/test_abi_cpu.py runs the reference's actual
-    wrapper over the same module in the build container (no reference tree on the GPU box)."""
+    a pyramid-sized fp32 case against the oracle (bit-exact forward).  tests/test_abi_cpu.py replays the calls recorded
+    from the reference's actual wrapper (tests/golden/mmcv_wrapper_calls.json) against the same module."""
     from gpt4roi_b200 import mmcv_ext
     ext = mmcv_ext.make_module()
     kat = load_kat()
