@@ -45,14 +45,7 @@ void set_sm_reserve_impl(int n) { g_sm_reserve = n < 0 ? 0 : n; }
 // sequence writes them -- true for the decode step, not for arbitrary callers (a cast or an optimizer kernel may
 // directly precede a small GEMM).
 static int g_pdl_on = 0;
-int pdl_mode() {
-  static int v = -1;
-  if (v < 0) {
-    const char* e = getenv("G4R_PDL");
-    v = !e ? 1 : (e[0] == '0' ? 0 : (e[0] == '2' ? 2 : 1));
-  }
-  return g_pdl_on ? v : 0;
-}
+bool pdl_on() { return g_pdl_on != 0; }
 
 }  // namespace g4r
 
@@ -69,5 +62,5 @@ extern "C" int g4r_set_sm_reserve(int n_sms) {
 }
 
 extern "C" const char* g4r_last_error(void) { return g4r::g_err; }
-extern "C" int g4r_version(void) { return 1000; }
+extern "C" int g4r_version(void) { return 1001; }
 extern "C" int g4r_built_arch(void) { return 100; }

@@ -68,8 +68,7 @@ template <int D, bool CAUSAL>
 __global__ void __launch_bounds__(kAttnThreads)
 flash_attn_fwd(const __nv_bfloat16* __restrict__ Q, const __nv_bfloat16* __restrict__ K,
                const __nv_bfloat16* __restrict__ V, __nv_bfloat16* __restrict__ O, long long ld, long long bs,
-               long long ldo, long long bso, int L, float scale, const int* __restrict__ seqlens,
-               float* __restrict__ lse_out /* optional [B, H, L]: log-sum-exp of the scaled scores (training) */) {
+               long long ldo, long long bso, int L, float scale, const int* __restrict__ seqlens) {
   extern __shared__ __align__(128) uint8_t smem_attn[];
   __nv_bfloat16* sQ = reinterpret_cast<__nv_bfloat16*>(smem_attn);
   __nv_bfloat16* sK = sQ + kBM * D;       // 2 buffers
@@ -214,8 +213,6 @@ flash_attn_fwd(const __nv_bfloat16* __restrict__ Q, const __nv_bfloat16* __restr
     const int qrow = q0 + warp * 16 + g + r * 8;
     if (qrow >= L) continue;
     const float inv = 1.f / l_run[r];
-    if (lse_out != nullptr && t == 0)
-      lse_out[((long long)b * gridDim.y + h) * L + qrow] = m_run[r] * scale + logf(l_run[r]);
 #pragma unroll
     for (int i = 0; i < D / 8; i++) {
       const uint32_t pk = pack_bf16(o[i][2 * r] * inv, o[i][2 * r + 1] * inv);
@@ -227,7 +224,7 @@ flash_attn_fwd(const __nv_bfloat16* __restrict__ Q, const __nv_bfloat16* __restr
 template <int D, bool CAUSAL>
 static int launch_attn(const void* q, const void* k, const void* v, void* o, long long ld, long long bs,
                        long long ldo, long long bso, int B, int H, int L, float scale, const int* seqlens,
-                       cudaStream_t st, float* lse = nullptr) {
+                       cudaStream_t st) {
   const int smem = (kBM * D + 4 * kBN * D) * 2;
   static bool set = false;
   auto kern = flash_attn_fwd<D, CAUSAL>;
@@ -237,7 +234,7 @@ static int launch_attn(const void* q, const void* k, const void* v, void* o, lon
   }
   dim3 grid((L + kBM - 1) / kBM, H, B);
   kern<<<grid, kAttnThreads, smem, st>>>((const __nv_bfloat16*)q, (const __nv_bfloat16*)k,
-                                          (const __nv_bfloat16*)v, (__nv_bfloat16*)o, ld, bs, ldo, bso, L, scale, seqlens, lse);
+                                          (const __nv_bfloat16*)v, (__nv_bfloat16*)o, ld, bs, ldo, bso, L, scale, seqlens);
   G4R_LAUNCH_CHECK("flash_attn_fwd");
   return G4R_OK;
 }
@@ -246,38 +243,18 @@ static int launch_attn(const void* q, const void* k, const void* v, void* o, lon
 
 using namespace G4R_NS;
 
-static int attention_impl(const void* q, const void* k, const void* v, void* out, long long ld, long long bs,
-                          long long ldo, long long bso, int B, int H, int L, int head_dim, int causal, float scale,
-                          const int* seqlens, float* lse, void* stream);
-
 extern "C" int g4r_attention_bf16(const void* q, const void* k, const void* v, void* out, long long ld,
                                   long long bs, long long ldo, long long bso, int B, int H, int L,
                                   int head_dim, int causal, float scale, const int* seqlens, void* stream) {
-  return attention_impl(q, k, v, out, ld, bs, ldo, bso, B, H, L, head_dim, causal, scale, seqlens, nullptr, stream);
-}
-
-// Training forward: same kernel, additionally writes lse[B, H, L] (fp32) for g4r_attention_bwd_bf16.
-#if G4R_BF16_ONLY   // training-step only: no fp16 twin
-extern "C" int g4r_attention_fwd_lse_bf16(const void* q, const void* k, const void* v, void* out, long long ld,
-                                          long long bs, long long ldo, long long bso, int B, int H, int L,
-                                          int head_dim, int causal, float scale, float* lse, void* stream) {
-  G4R_REQUIRE(lse, "attention_fwd_lse: lse is NULL");
-  return attention_impl(q, k, v, out, ld, bs, ldo, bso, B, H, L, head_dim, causal, scale, nullptr, lse, stream);
-}
-#endif
-
-static int attention_impl(const void* q, const void* k, const void* v, void* out, long long ld, long long bs,
-                          long long ldo, long long bso, int B, int H, int L, int head_dim, int causal, float scale,
-                          const int* seqlens, float* lse, void* stream) {
   G4R_REQUIRE(q && k && v && out && B > 0 && H > 0 && L > 0, "attention: bad arguments");
   G4R_REQUIRE(head_dim == 64 || head_dim == 128, "attention: head_dim %d (64 or 128)", head_dim);
   G4R_REQUIRE(ld % 8 == 0 && bs % 8 == 0 && ldo % 2 == 0 && bso % 2 == 0, "attention: strides must keep 16-byte row alignment");
   G4R_REQUIRE((((uintptr_t)q | (uintptr_t)k | (uintptr_t)v) & 15) == 0 && ((uintptr_t)out & 3) == 0, "attention: misaligned pointers");
   cudaStream_t st = (cudaStream_t)stream;
   if (head_dim == 64) {
-    return causal ? launch_attn<64, true>(q, k, v, out, ld, bs, ldo, bso, B, H, L, scale, seqlens, st, lse)
-                  : launch_attn<64, false>(q, k, v, out, ld, bs, ldo, bso, B, H, L, scale, seqlens, st, lse);
+    return causal ? launch_attn<64, true>(q, k, v, out, ld, bs, ldo, bso, B, H, L, scale, seqlens, st)
+                  : launch_attn<64, false>(q, k, v, out, ld, bs, ldo, bso, B, H, L, scale, seqlens, st);
   }
-  return causal ? launch_attn<128, true>(q, k, v, out, ld, bs, ldo, bso, B, H, L, scale, seqlens, st, lse)
-                : launch_attn<128, false>(q, k, v, out, ld, bs, ldo, bso, B, H, L, scale, seqlens, st, lse);
+  return causal ? launch_attn<128, true>(q, k, v, out, ld, bs, ldo, bso, B, H, L, scale, seqlens, st)
+                : launch_attn<128, false>(q, k, v, out, ld, bs, ldo, bso, B, H, L, scale, seqlens, st);
 }

@@ -2,7 +2,7 @@
 // the reference gets it from autograd through transformers' eager LLaMA attention, modeling_llama.py:199-222).
 //
 // Inputs: packed qkv rows [B*L, 3*H*D] (after RoPE), the forward output O, its log-sum-exp rows
-// (g4r_attention_fwd_lse_bf16) and dO.  Output: packed dqkv rows (dQ | dK | dV), bf16.
+// (g4r_attention_tc_lse_bf16) and dO.  Output: packed dqkv rows (dQ | dK | dV), bf16.
 // Two kernels, both recomputing S = Q K^T from the saved LSE (no [L, L] tensor is ever stored) and both
 // free of atomics, so gradients are bitwise reproducible:
 //   attn_bwd_dq : one CTA per 64-query block, loops over the key blocks it can see:

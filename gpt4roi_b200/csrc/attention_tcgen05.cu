@@ -24,6 +24,10 @@
 namespace G4R_NS {
 
 constexpr int kFaBM = 128;
+// keys per block.  64 keeps a CTA at 112 KB of shared memory and 256 TMEM columns (D=128), so TWO CTAs share an SM:
+// one CTA's prologue / epilogue overlaps the other's MMAs and 8 softmax warps instead of 4 hide the tcgen05.ld / MUFU
+// latencies.
+constexpr int kFaBN = 64;
 constexpr int kFaThreads = 256;
 constexpr int kAtomBytes = 128 * 128;  // [128 rows][64 bf16] swizzle-128B atom (Q, P)
 
@@ -51,20 +55,16 @@ __device__ __forceinline__ void tmem_st_wait() { asm volatile("tcgen05.wait::st.
 
 using ptx::make_smem_desc_mn_sw128;  // V tile [keys][d] (d contiguous) is an MN-major B operand
 
-// BN = keys per block.  BN=64 keeps a CTA at 112 KB of shared memory and 256 TMEM columns (D=128), so
-// TWO CTAs share an SM: one CTA's prologue / epilogue overlaps the other's MMAs and 8 softmax warps
-// instead of 4 hide the tcgen05.ld / MUFU latencies.
-template <int D, int BN, bool CAUSAL>
-__global__ void __launch_bounds__(kFaThreads, (BN == 64 ? 2 : 1))
+template <int D, bool CAUSAL>
+__global__ void __launch_bounds__(kFaThreads, 2)
 fa_fwd_tcgen05(const __grid_constant__ CUtensorMap tm_q, const __grid_constant__ CUtensorMap tm_k,
                const __grid_constant__ CUtensorMap tm_v, const __grid_constant__ FaParams p) {
-  constexpr int kFaBN = BN;
   constexpr int ATOMS = D / 64;
-  constexpr int Q_BYTES = ATOMS * kAtomBytes;     // Q tile: 128 rows x D
-  constexpr int KV_ATOM = BN * 128;               // [BN keys][64 bf16]
-  constexpr int TILE_BYTES = ATOMS * KV_ATOM;     // K / V tile: BN rows x D
-  constexpr int P_BYTES = (BN / 64) * kAtomBytes; // P: 128 x BN keys
-  constexpr int TMEM_COLS = (2 * BN + D) <= 256 ? 256 : 512;
+  constexpr int Q_BYTES = ATOMS * kAtomBytes;        // Q tile: 128 rows x D
+  constexpr int KV_ATOM = kFaBN * 128;               // [kFaBN keys][64 bf16]
+  constexpr int TILE_BYTES = ATOMS * KV_ATOM;        // K / V tile: kFaBN rows x D
+  constexpr int P_BYTES = (kFaBN / 64) * kAtomBytes; // P: 128 x kFaBN keys
+  constexpr int TMEM_COLS = (2 * kFaBN + D) <= 256 ? 256 : 512;
   extern __shared__ __align__(1024) uint8_t smem[];
   uint8_t* sQ = smem;
   uint8_t* sK = sQ + Q_BYTES;          // 2 stages
@@ -344,12 +344,12 @@ static int make_tmap_rows(CUtensorMap* m, const void* base, long long cols, long
   return G4R_OK;
 }
 
-template <int D, int BN, bool CAUSAL>
+template <int D, bool CAUSAL>
 static int launch_fa(const CUtensorMap& tq, const CUtensorMap& tk, const CUtensorMap& tv, const FaParams& p, int B,
                      cudaStream_t st) {
-  constexpr int smem = (D / 64) * kAtomBytes + 4 * (D / 64) * BN * 128 + (BN / 64) * kAtomBytes + 256;
+  constexpr int smem = (D / 64) * kAtomBytes + 4 * (D / 64) * kFaBN * 128 + (kFaBN / 64) * kAtomBytes + 256;
   static bool set = false;
-  auto kern = fa_fwd_tcgen05<D, BN, CAUSAL>;
+  auto kern = fa_fwd_tcgen05<D, CAUSAL>;
   if (!set) {
     G4R_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
     set = true;
@@ -377,20 +377,13 @@ static int attention_tc_impl(const void* q, const void* k, const void* v, void* 
   CUtensorMap tq, tk, tv;
   const long long cols = (long long)H * head_dim, rows = (long long)B * L;
   int rc;
-  static int bn = 0;
-  if (!bn) {
-    const char* e = getenv("G4R_ATTN_BN");
-    bn = (e && atoi(e) == 128) ? 128 : 64;
-  }
   if ((rc = make_tmap_rows(&tq, q, cols, rows, ld, 128))) return rc;
-  if ((rc = make_tmap_rows(&tk, k, cols, rows, ld, bn))) return rc;
-  if ((rc = make_tmap_rows(&tv, v, cols, rows, ld, bn))) return rc;
+  if ((rc = make_tmap_rows(&tk, k, cols, rows, ld, kFaBN))) return rc;
+  if ((rc = make_tmap_rows(&tv, v, cols, rows, ld, kFaBN))) return rc;
   FaParams p{(__nv_bfloat16*)out, ldo, bso, L, H, scale, seqlens, lse};
   cudaStream_t st = (cudaStream_t)stream;
-#define G4R_FA(DD, BB) (causal ? launch_fa<DD, BB, true>(tq, tk, tv, p, B, st) : launch_fa<DD, BB, false>(tq, tk, tv, p, B, st))
-  if (head_dim == 64) return bn == 128 ? G4R_FA(64, 128) : G4R_FA(64, 64);
-  return bn == 128 ? G4R_FA(128, 128) : G4R_FA(128, 64);
-#undef G4R_FA
+  if (head_dim == 64) return causal ? launch_fa<64, true>(tq, tk, tv, p, B, st) : launch_fa<64, false>(tq, tk, tv, p, B, st);
+  return causal ? launch_fa<128, true>(tq, tk, tv, p, B, st) : launch_fa<128, false>(tq, tk, tv, p, B, st);
 }
 
 extern "C" int g4r_attention_tc_bf16(const void* q, const void* k, const void* v, void* out, long long ld,

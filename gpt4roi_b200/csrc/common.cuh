@@ -56,17 +56,17 @@ int sm_budget();  // num_sms() minus the reserve of g4r_set_sm_reserve (grid siz
 // visible.  Everything read BEFORE pdl_wait() must be constant for the step (weights); everything the predecessor
 // produced is read after it, through ordinary (coherent) loads.  Every kernel launched this way must execute
 // pdl_wait() before it exits, so completion stays transitive along the chain.
-//   pdl_mode(): 0 unless the caller has switched the chain on with g4r_set_pdl(1) (the decode step does; nothing else
-//   may -- see api_common.cu); then env G4R_PDL -- 0 off (plain stream order), 1 (default) dependents released once
-//   this kernel's own inputs are ready (one kernel of look-ahead), 2 dependents released at kernel start.
-int pdl_mode();
+//   pdl_on(): false unless the caller has switched the chain on with g4r_set_pdl(1) (the decode step does; nothing
+//   else may -- see api_common.cu).  Off, the kernels launch in plain stream order and pdl_sync() is a no-op.
+bool pdl_on();
 __device__ __forceinline__ void pdl_wait() { asm volatile("griddepcontrol.wait;" ::: "memory"); }
 __device__ __forceinline__ void pdl_release() { asm volatile("griddepcontrol.launch_dependents;" ::: "memory"); }
-// prologue of a PDL-aware kernel, after the loads that do not depend on the predecessor have been issued
-__device__ __forceinline__ void pdl_sync(int mode) {
-  if (mode == 2) pdl_release();
+// prologue of a PDL-aware kernel, after the loads that do not depend on the predecessor have been issued: dependents
+// are released once this kernel's own inputs are ready (one kernel of look-ahead; releasing them at kernel start
+// measured 3.36 vs 3.34 ms per decode step, profiles/r2_decode_pdl_depth.md)
+__device__ __forceinline__ void pdl_sync() {
   pdl_wait();
-  if (mode != 2) pdl_release();
+  pdl_release();
 }
 
 template <typename... KArgs, typename... Args>
@@ -82,7 +82,7 @@ static inline cudaError_t launch_pdl(void (*kern)(KArgs...), dim3 grid, dim3 blo
   attr[n].id = cudaLaunchAttributeClusterDimension;
   attr[n].val.clusterDim.x = cluster.x; attr[n].val.clusterDim.y = cluster.y; attr[n].val.clusterDim.z = cluster.z;
   n++;
-  if (pdl_mode() != 0) {
+  if (pdl_on()) {
     attr[n].id = cudaLaunchAttributeProgrammaticStreamSerialization;
     attr[n].val.programmaticStreamSerializationAllowed = 1;
     n++;

@@ -40,11 +40,11 @@ template <int D>
 __global__ void __launch_bounds__(256)
 decode_attention_bf16(const __nv_bfloat16* q, long long ldq, const __nv_bfloat16* kc, const __nv_bfloat16* vc,
                       __nv_bfloat16* out, long long ldo, int H, int kv_len, const int* __restrict__ pos_dev, int Lmax,
-                      float scale, int per_max, int pdl) {
+                      float scale, int per_max) {
   // Programmatic dependent launch (common.cuh): q and the newest K/V row come from the q|k|v GEMM that precedes this
   // kernel in the decode step, so there is nothing to fetch ahead; the launch itself and the prologue overlap its tail.
   // q / kc / vc carry no __restrict__: their loads must stay on the coherent path.
-  pdl_sync(pdl);
+  pdl_sync();
   static_assert(D == 128 || D == 64, "head_dim");
   constexpr int LPR = D / 8;          // lanes per row (16 or 8)
   constexpr int RPW = 32 / LPR;       // rows per warp instruction (2 or 4)
@@ -219,7 +219,7 @@ static int launch_decode_attention(const void* q, long long ldq, const void* kca
   }
   G4R_CUDA(launch_pdl(decode_attention_bf16<D>, dim3(H, B, S), dim3(256), smem, st, dim3(1, 1, S),
                       (const __nv_bfloat16*)q, ldq, (const __nv_bfloat16*)kcache, (const __nv_bfloat16*)vcache,
-                      (__nv_bfloat16*)out, ldo, H, kv_len, pos_dev, Lmax, scale, per_max, pdl_mode()));
+                      (__nv_bfloat16*)out, ldo, H, kv_len, pos_dev, Lmax, scale, per_max));
   return G4R_OK;
 }
 

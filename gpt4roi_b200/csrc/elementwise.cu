@@ -149,7 +149,7 @@ template <bool RMS, int PER>
 __global__ void __launch_bounds__(256)
 norm_row_cta_bf16(const __nv_bfloat16* x, long long ldx, const __nv_bfloat16* __restrict__ w,
                   const __nv_bfloat16* __restrict__ b, __nv_bfloat16* out, long long ldo, int D,
-                  float eps, int pdl) {
+                  float eps) {
   __shared__ float red[8];
   __shared__ float stat;
   const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
@@ -162,7 +162,7 @@ norm_row_cta_bf16(const __nv_bfloat16* x, long long ldx, const __nv_bfloat16* __
   uint4 wraw[PER];
 #pragma unroll
   for (int i = 0; i < PER; i++) wraw[i] = tid + i * 256 < nvec ? __ldg(wv + tid + i * 256) : make_uint4(0, 0, 0, 0);
-  pdl_sync(pdl);
+  pdl_sync();
   float v[PER][8];
   float sum = 0.f, sumsq = 0.f;
 #pragma unroll
@@ -234,7 +234,7 @@ static int launch_norm(const void* x, long long ldx, const void* w, const void* 
 #define G4R_NORM_ROW_CASE(PR)                                                                              \
   G4R_CUDA(launch_pdl(norm_row_cta_bf16<RMS, PR>, dim3(M), dim3(256), 0, st, dim3(1, 1, 1),                \
                       (const __nv_bfloat16*)x, ldx, (const __nv_bfloat16*)w, (const __nv_bfloat16*)b,     \
-                      (__nv_bfloat16*)out, ldo, D, eps, pdl_mode()))
+                      (__nv_bfloat16*)out, ldo, D, eps))
     if (per <= 1) G4R_NORM_ROW_CASE(1);
     else if (per <= 2) G4R_NORM_ROW_CASE(2);
     else G4R_NORM_ROW_CASE(4);

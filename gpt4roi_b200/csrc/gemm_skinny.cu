@@ -16,13 +16,8 @@
 // k16 steps from ONE 16-byte load at physical k0 + 8t .. 8t+7, from the weight row and from the
 // activation row alike -- no shuffles, no shared-memory staging, full-sector global loads.
 //
-// Optional split-K over a thread-block cluster (G4R_SKINNY_CTAS=<target CTA count>): the KS CTAs of a
-// cluster (gridDim.y) share one weight-row tile and interleave its k-blocks; partial sums meet in rank 0
-// through distributed shared memory.  Measured slower than KS=1 on B200 (profiles/r1_decode_kernels.md),
-// so it is off by default; bytes in flight per SM come from 16-warp CTAs on the narrow-N shapes instead.
-// Deterministic: partial sums of the warps and of the cluster ranks are added in fixed order.
+// Deterministic: the partial sums of the warps are added in a fixed order.
 #include "common.cuh"
-#include <cooperative_groups.h>
 #include "act_type.cuh"   // bf16 as written; fp16 twin with -DG4R_ACT_HALF
 
 namespace G4R_NS {
@@ -40,11 +35,9 @@ struct SkinnyParams {
   const __nv_bfloat16* rope_cos; const __nv_bfloat16* rope_sin;
   int rope_cols, rope_L, rope_pos0;
   const int* rope_pos_dev;
-  // decode-step fusions (all optional):
-  const __nv_bfloat16* norm_w; float norm_eps;   // RMSNorm of the activation rows before the product (K = hidden)
+  // decode-step fusion (optional):
   __nv_bfloat16* kcache; __nv_bfloat16* vcache;  // [M, cache_lmax, cache_hd]: k / v columns are also written at `pos`
   int cache_lmax, cache_hd;
-  int pdl;   // pdl_mode() of the launch (common.cuh)
 };
 
 // weights: constant for the lifetime of the step, read exactly once.  volatile: the first block is issued BEFORE
@@ -75,35 +68,16 @@ __device__ __forceinline__ float bf16r(float x) { return __bfloat162float(__floa
 // MT: 16-row weight tiles per CTA (1 or 2); MB: 8-row activation blocks (1: M<=8, 2: M<=16);
 // ROPE: the two tiles are 64 rows apart (dims d and d+64 of one 128-dim head) so the rotation has
 // both partners in the CTA.
-// RMSNorm folded into the activation fragment (LlamaRMSNorm, modeling_llama.py:53-67, with the rounding points of
-// norm_rows_bf16: bf16(x * rstd), times the bf16 weight, rounded to bf16): 8 packed bf16 -> 8 packed bf16.
-__device__ __forceinline__ uint4 norm8(const uint4& x, const uint4& w, float rstd) {
-  const __nv_bfloat162* xh = reinterpret_cast<const __nv_bfloat162*>(&x);
-  const __nv_bfloat162* wh = reinterpret_cast<const __nv_bfloat162*>(&w);
-  uint4 o;
-  __nv_bfloat162* oh = reinterpret_cast<__nv_bfloat162*>(&o);
-#pragma unroll
-  for (int j = 0; j < 4; j++) {
-    const float2 xf = __bfloat1622float2(xh[j]), wf = __bfloat1622float2(wh[j]);
-    oh[j] = __floats2bfloat162_rn(wf.x * bf16r(xf.x * rstd), wf.y * bf16r(xf.y * rstd));
-  }
-  return o;
-}
-
 // DEPTH: k-blocks each warp keeps in flight (register double buffering): with DEPTH = 2 a warp that owns two k-blocks
 // (o_proj: K = 4096 over 16 warps) requests its whole share before the first MMA -- one HBM latency instead of two.
-template <int MT, int MB, int WARPS, bool ROPE, bool NORM = false, int DEPTH = 1>
-__global__ void __launch_bounds__(WARPS * 32)
+// DEPTH = 2 relies on 2 CTAs per SM (see gemm_skinny_run), i.e. <= 128 registers; the launch bound holds ptxas to it.
+template <int MT, int MB, int WARPS, bool ROPE, int DEPTH = 1>
+__global__ void __launch_bounds__(WARPS * 32, DEPTH == 2 ? 2 : 0)
 gemm_skinny_bf16(const SkinnyParams p) {
   constexpr int KB = 128;        // k per warp iteration: 4 sub-blocks of 32 (one 16-byte load per row each)
   constexpr int NT = MT * 16;
   constexpr int MC = MB * 8;
   __shared__ float red[WARPS][NT][MC + 1];
-  __shared__ float ctot[NT][MC];   // this CTA's k-slice total, read by cluster rank 0
-  __shared__ float s_rstd[MC];
-  namespace cg = cooperative_groups;
-  cg::cluster_group cluster = cg::this_cluster();
-  const int KS = (int)cluster.num_blocks(), rank = (int)cluster.block_rank();
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31, g = lane >> 2, t = lane & 3;
   const int tile_stride = ROPE ? 64 : 16;
   const int n_base = ROPE ? (int)(blockIdx.x >> 2) * 128 + (int)(blockIdx.x & 3) * 16 : (int)blockIdx.x * NT;
@@ -137,8 +111,8 @@ gemm_skinny_bf16(const SkinnyParams p) {
 
   // The first weight block of every warp does not depend on the predecessor kernel: issue it, then wait for the
   // predecessor (programmatic dependent launch, common.cuh) -- its tail and this kernel's ramp-up overlap.
-  const int kstep = KS * WARPS * KB;
-  int k0 = (rank * WARPS + warp) * KB;
+  constexpr int kstep = WARPS * KB;
+  int k0 = warp * KB;
   uint4 a[DEPTH][4][MT][2];
   auto load_w = [&](uint4 (&aw)[4][MT][2], int kb) {
 #pragma unroll
@@ -159,30 +133,7 @@ gemm_skinny_bf16(const SkinnyParams p) {
 #pragma unroll
   for (int d = 0; d < DEPTH; d++)
     if (k0 + d * kstep < p.K) load_w(a[d], k0 + d * kstep);
-  pdl_sync(p.pdl);
-
-  if constexpr (NORM) {
-    // rstd of every activation row, recomputed by each CTA (M <= 16 rows of K bf16 from L2): warp w takes rows w, w+WARPS, ..
-    for (int m = warp; m < MC; m += WARPS) {
-      float ss = 0.f;
-      if (m < p.M) {
-        const __nv_bfloat16* xr = p.A + (long long)m * p.lda;
-        for (int k = lane * 8; k < p.K; k += 256) {
-          const uint4 raw = ldg_act16(xr + k);
-          const __nv_bfloat162* h2 = reinterpret_cast<const __nv_bfloat162*>(&raw);
-#pragma unroll
-          for (int j = 0; j < 4; j++) { const float2 f = __bfloat1622float2(h2[j]); ss += f.x * f.x + f.y * f.y; }
-        }
-      }
-#pragma unroll
-      for (int o = 16; o > 0; o >>= 1) ss += __shfl_xor_sync(0xffffffffu, ss, o);
-      if (lane == 0) s_rstd[m] = rsqrtf(ss / p.K + p.norm_eps);
-    }
-    __syncthreads();
-  }
-  float rstd[MB];
-#pragma unroll
-  for (int i = 0; i < MB; i++) rstd[i] = NORM ? s_rstd[i * 8 + g] : 1.f;
+  pdl_sync();
 
   // activation fragments of a k-block; like the weights they are fetched DEPTH blocks ahead, so that all loads of a
   // block are issued back to back (left inside the loop body, ptxas strings them out between the dependent HMMAs)
@@ -196,11 +147,6 @@ gemm_skinny_bf16(const SkinnyParams p) {
       for (int i = 0; i < MB; i++) {
         const uint4 v = ldg_act16(xrow[i] + kk);   // rows >= M alias row 0; their outputs are never stored
         bx[s][i] = kok ? v : make_uint4(0, 0, 0, 0);
-      }
-      if constexpr (NORM) {
-        const uint4 w8 = __ldg(reinterpret_cast<const uint4*>(p.norm_w + kk + 8 * t));
-#pragma unroll
-        for (int i = 0; i < MB; i++) bx[s][i] = norm8(bx[s][i], w8, rstd[i]);
       }
     }
   };
@@ -238,21 +184,10 @@ gemm_skinny_bf16(const SkinnyParams p) {
       for (int c = 0; c < 4; c++) red[warp][j * 16 + g + 8 * (c >> 1)][i * 8 + 2 * t + (c & 1)] = acc[j][i][c];
   __syncthreads();
 
-  for (int e = threadIdx.x; e < NT * MC; e += WARPS * 32) {
-    const int r = e % NT, m = e / NT;
+  auto total = [&](int r, int m) {   // warps in fixed order: bitwise reproducible
     float v = 0.f;
 #pragma unroll
     for (int w = 0; w < WARPS; w++) v += red[w][r][m];
-    ctot[r][m] = v;
-  }
-  cluster.sync();
-  if (rank != 0) {
-    cluster.sync();   // stay resident until rank 0 has read this CTA's totals
-    return;
-  }
-  auto total = [&](int r, int m) {
-    float v = ctot[r][m];
-    for (int c = 1; c < KS; c++) v += (*cluster.map_shared_rank(&ctot, c))[r][m];
     return v;
   };
 
@@ -293,7 +228,6 @@ gemm_skinny_bf16(const SkinnyParams p) {
         }
       }
     }
-    cluster.sync();
     return;
   }
 
@@ -319,27 +253,11 @@ gemm_skinny_bf16(const SkinnyParams p) {
     if (p.residual != nullptr) v += __bfloat162float(p.residual[(long long)m * p.ldr + n]);
     p.D[(long long)m * p.ldd + n] = __float2bfloat16_rn(v);
   }
-  cluster.sync();
 }
 
-static int skinny_target_ctas() {
-  static int v = -1;
-  if (v < 0) {
-    const char* e = getenv("G4R_SKINNY_CTAS");
-    v = e ? atoi(e) : 0;   // default: no split-K (measured: cluster scheduling costs more than the tail it removes)
-  }
-  return v;
-}
-
-template <int MT, int MB, int WARPS, bool ROPE, bool NORM = false, int DEPTH = 1>
+template <int MT, int MB, int WARPS, bool ROPE, int DEPTH = 1>
 static int launch_skinny(const SkinnyParams& p, unsigned tiles, cudaStream_t st) {
-  // cluster split-K factor: enough CTAs for several waves, every warp keeps >= 1 k-block of 128
-  int ks = 1;
-  while (ks < 8 && (int)tiles * ks < skinny_target_ctas() && p.K >= 2 * ks * WARPS * 128) ks *= 2;
-  SkinnyParams q = p;
-  q.pdl = pdl_mode();
-  G4R_CUDA(launch_pdl(gemm_skinny_bf16<MT, MB, WARPS, ROPE, NORM, DEPTH>, dim3(tiles, ks, 1), dim3(WARPS * 32), 0, st,
-                      dim3(1, ks, 1), q));
+  G4R_CUDA(launch_pdl(gemm_skinny_bf16<MT, MB, WARPS, ROPE, DEPTH>, dim3(tiles), dim3(WARPS * 32), 0, st, dim3(1, 1, 1), p));
   return G4R_OK;
 }
 
@@ -353,63 +271,43 @@ static bool wide_prefers_8_warps(int tiles) {
   return waste(w8) < 0.95 * waste(w4);
 }
 
-// Called by gemm_impl (gemm_tcgen05.cu) when the shape qualifies; returns -1 when it does not.
+// Tile selection for both entry points: gemm_impl (gemm_tcgen05.cu) and g4r_decode_gemm_*.  Returns -1 when the shape
+// does not qualify.
+static int gemm_skinny_run(SkinnyParams p, cudaStream_t st) {
+  if (p.M > 16 || p.K % 32 != 0) return -1;
+  if (p.act == SK_ACT_SWIGLU && (p.N % 2 != 0)) return -1;
+  p.rope_L = p.rope_L > 0 ? p.rope_L : 1;
+  if (p.rope_cos != nullptr) {
+    if (p.N % 128 != 0) return -1;
+    const unsigned grid = (unsigned)(p.N / 128) * 4;
+    return p.M <= 8 ? launch_skinny<2, 1, 4, true>(p, grid, st) : launch_skinny<2, 2, 4, true>(p, grid, st);
+  }
+  // 32-row tiles halve the activation re-reads; use them once they still give >= 2 CTAs per SM
+  const bool wide = (p.N + 31) / 32 >= 2 * num_sms();
+  if (wide) {
+    const unsigned grid = (unsigned)((p.N + 31) / 32);
+    if (p.M > 8) return launch_skinny<2, 2, 4, false>(p, grid, st);
+    return wide_prefers_8_warps((int)grid) ? launch_skinny<2, 1, 8, false>(p, grid, st) : launch_skinny<2, 1, 4, false>(p, grid, st);
+  }
+  const unsigned grid = (unsigned)((p.N + 15) / 16);
+  // 16-row tiles give few CTAs (N/16 = 256 for the 4096-row projections).  M <= 8: 8 warps with two k-blocks in flight
+  // each (128 registers -> 2 CTAs per SM, so all 256 CTAs are resident at once and request half the matrix up front):
+  // o_proj 11.4 -> 8.4 us, down_proj 21.5 -> 17.8 us (B200, profiles/r2_decode_pdl_depth.md).  M <= 16: 16 warps.
+  return p.M <= 8 ? launch_skinny<1, 1, 8, false, 2>(p, grid, st) : launch_skinny<1, 2, 16, false>(p, grid, st);
+}
+
+// Called by gemm_impl (gemm_tcgen05.cu) for M <= 16; returns -1 when the shape does not qualify.
 int gemm_skinny_dispatch(const void* A, long long lda, const void* B, long long ldb, void* D, long long ldd, int M,
                          int N, int K, const void* bias, int bias_f32, const void* residual, long long ldr, int act,
                          const void* rope_cos, const void* rope_sin, int rope_cols, int rope_L, int rope_pos0,
                          const int* rope_pos_dev, void* stream) {
-  if (M > 16 || K % 32 != 0) return -1;
-  if (act == SK_ACT_SWIGLU && (N % 2 != 0)) return -1;
   SkinnyParams p{};
   p.A = (const __nv_bfloat16*)A; p.lda = lda; p.W = (const __nv_bfloat16*)B; p.ldb = ldb;
   p.D = (__nv_bfloat16*)D; p.ldd = ldd; p.M = M; p.N = N; p.K = K;
   p.bias = bias; p.bias_f32 = bias_f32; p.residual = (const __nv_bfloat16*)residual; p.ldr = ldr; p.act = act;
   p.rope_cos = (const __nv_bfloat16*)rope_cos; p.rope_sin = (const __nv_bfloat16*)rope_sin;
-  p.rope_cols = rope_cols; p.rope_L = rope_L > 0 ? rope_L : 1; p.rope_pos0 = rope_pos0; p.rope_pos_dev = rope_pos_dev;
-  cudaStream_t st = (cudaStream_t)stream;
-  if (rope_cos != nullptr) {
-    if (N % 128 != 0) return -1;
-    const unsigned grid = (unsigned)(N / 128) * 4;
-    return M <= 8 ? launch_skinny<2, 1, 4, true>(p, grid, st) : launch_skinny<2, 2, 4, true>(p, grid, st);
-  }
-  // 32-row tiles halve the activation re-reads; use them once they still give >= 2 CTAs per SM
-  const bool wide = (N + 31) / 32 >= 2 * num_sms();
-  if (wide) {
-    const unsigned grid = (unsigned)((N + 31) / 32);
-    if (M > 8) return launch_skinny<2, 2, 4, false>(p, grid, st);
-    return wide_prefers_8_warps((int)grid) ? launch_skinny<2, 1, 8, false>(p, grid, st) : launch_skinny<2, 1, 4, false>(p, grid, st);
-  }
-  const unsigned grid = (unsigned)((N + 15) / 16);
-  // 16-row tiles give few CTAs (N/16 = 256 for the 4096-row projections).  M <= 8: 8 warps with two k-blocks in flight
-  // each (128 registers -> 2 CTAs per SM, so all 256 CTAs are resident at once and request half the matrix up front):
-  // o_proj 11.4 -> 8.4 us, down_proj 21.5 -> 17.8 us (B200, profiles/r2_decode_pdl_depth.md).  M <= 16: 16 warps.
-  return M <= 8 ? launch_skinny<1, 1, 8, false, false, 2>(p, grid, st) : launch_skinny<1, 2, 16, false>(p, grid, st);
-}
-
-// Decode-step fused entry (M <= 16): [RMSNorm ->] GEMM [-> RoPE + KV-cache write | SwiGLU | residual].
-int gemm_skinny_fused(const SkinnyParams& p0, cudaStream_t st) {
-  SkinnyParams p = p0;
-  if (p.M > 16 || p.K % 32 != 0) return -1;
-  p.rope_L = p.rope_L > 0 ? p.rope_L : 1;
-  const bool norm = p.norm_w != nullptr;
-  if (norm && p.K % 256 != 0) return -1;
-  if (p.rope_cos != nullptr) {
-    if (p.N % 128 != 0) return -1;
-    const unsigned grid = (unsigned)(p.N / 128) * 4;
-    if (norm) return p.M <= 8 ? launch_skinny<2, 1, 4, true, true>(p, grid, st) : launch_skinny<2, 2, 4, true, true>(p, grid, st);
-    return p.M <= 8 ? launch_skinny<2, 1, 4, true>(p, grid, st) : launch_skinny<2, 2, 4, true>(p, grid, st);
-  }
-  if (p.act == SK_ACT_SWIGLU && (p.N % 2 != 0)) return -1;
-  const bool wide = (p.N + 31) / 32 >= 2 * num_sms();
-  if (wide) {
-    const unsigned grid = (unsigned)((p.N + 31) / 32);
-    if (norm) return p.M <= 8 ? launch_skinny<2, 1, 4, false, true>(p, grid, st) : launch_skinny<2, 2, 4, false, true>(p, grid, st);
-    if (p.M > 8) return launch_skinny<2, 2, 4, false>(p, grid, st);
-    return wide_prefers_8_warps((int)grid) ? launch_skinny<2, 1, 8, false>(p, grid, st) : launch_skinny<2, 1, 4, false>(p, grid, st);
-  }
-  const unsigned grid = (unsigned)((p.N + 15) / 16);
-  if (norm) return p.M <= 8 ? launch_skinny<1, 1, 16, false, true>(p, grid, st) : launch_skinny<1, 2, 16, false, true>(p, grid, st);
-  return p.M <= 8 ? launch_skinny<1, 1, 8, false, false, 2>(p, grid, st) : launch_skinny<1, 2, 16, false>(p, grid, st);
+  p.rope_cols = rope_cols; p.rope_L = rope_L; p.rope_pos0 = rope_pos0; p.rope_pos_dev = rope_pos_dev;
+  return gemm_skinny_run(p, (cudaStream_t)stream);
 }
 
 }  // namespace g4r
@@ -417,8 +315,7 @@ int gemm_skinny_fused(const SkinnyParams& p0, cudaStream_t st) {
 using namespace G4R_NS;
 
 extern "C" int g4r_decode_gemm_bf16(const void* x, long long ldx, const void* W, long long ldw, void* out, long long ldo,
-                                    int M, int N, int K, const void* norm_w, float norm_eps, int act, const void* residual,
-                                    long long ldr, const void* rope_cos, const void* rope_sin, int rope_cols, int pos0,
+                                    int M, int N, int K, int act, const void* residual, long long ldr, const void* rope_cos, const void* rope_sin, int rope_cols, int pos0,
                                     const int* pos_dev, void* kcache, void* vcache, int cache_lmax, int cache_hd,
                                     void* stream) {
   G4R_REQUIRE(x && W && out && M > 0 && M <= 16 && N > 0 && K > 0, "decode_gemm: M must be 1..16 (got %d)", M);
@@ -433,9 +330,8 @@ extern "C" int g4r_decode_gemm_bf16(const void* x, long long ldx, const void* W,
   p.residual = (const __nv_bfloat16*)residual; p.ldr = ldr; p.act = act;
   p.rope_cos = (const __nv_bfloat16*)rope_cos; p.rope_sin = (const __nv_bfloat16*)rope_sin;
   p.rope_cols = rope_cols; p.rope_L = 1; p.rope_pos0 = pos0; p.rope_pos_dev = pos_dev;
-  p.norm_w = (const __nv_bfloat16*)norm_w; p.norm_eps = norm_eps;
   p.kcache = (__nv_bfloat16*)kcache; p.vcache = (__nv_bfloat16*)vcache; p.cache_lmax = cache_lmax; p.cache_hd = cache_hd;
-  const int rc = gemm_skinny_fused(p, (cudaStream_t)stream);
+  const int rc = gemm_skinny_run(p, (cudaStream_t)stream);
   if (rc == -1) { set_error("decode_gemm: shape not supported (M=%d N=%d K=%d)", M, N, K); return G4R_EUNSUPPORTED; }
   return rc;
 }

@@ -756,14 +756,9 @@ static int launch_gemm_2sm(const CUtensorMap& ta, const CUtensorMap& tb, const G
 // B200, round 2 (profiles/r2_gemm_2sm_ab.md): the 2-CTA kernel beats the 1-CTA kernel on every LLaMA shape
 // (qkv 1416 vs 1317, o 1322 vs 1253, gate/up 1470 vs 1415, down 1413 vs 1305 TFLOP/s under ncu) although
 // M = B*L = 5648 rows leave a 94 %-empty last 256-row pair, and runs the convs at 1.58 PFLOP/s; whole step 106.0 vs
-// 107.4 ms.  G4R_GEMM_2SM=0 disables it everywhere, =2 restores the round-1 policy (convs only).
-static bool use_2sm(int N, int m_tiles, int k_splits, bool conv) {
-  static int env = -1;
-  if (env < 0) {
-    const char* e = getenv("G4R_GEMM_2SM");
-    env = !e ? 1 : (e[0] == '0' ? 0 : (e[0] == '2' ? 2 : 1));
-  }
-  if (env == 0 || (env == 2 && !conv) || N <= 128 || m_tiles < 2) return false;
+// 107.4 ms.
+static bool use_2sm(int N, int m_tiles, int k_splits) {
+  if (N <= 128 || m_tiles < 2) return false;
   const long pairs = (long)((m_tiles + 1) / 2) * ((N + 255) / 256) * k_splits;
   return pairs >= num_sms() / 2;
 }
@@ -808,11 +803,6 @@ int gemm_skinny_dispatch(const void* A, long long lda, const void* B, long long 
                          int N, int K, const void* bias, int bias_f32, const void* residual, long long ldr, int act,
                          const void* rope_cos, const void* rope_sin, int rope_cols, int rope_L, int rope_pos0,
                          const int* rope_pos_dev, void* stream);
-}
-static bool skinny_enabled() {
-  static int v = -1;
-  if (v < 0) { const char* e = getenv("G4R_SKINNY"); v = (e && e[0] == '0') ? 0 : 1; }
-  return v == 1;
 }
 
 extern "C" int g4r_gemm_bf16_ex(const void* A, long long lda, const void* B, long long ldb, void* D,
@@ -860,10 +850,8 @@ extern "C" int g4r_gemm_bf16_t(const void* A, long long lda, int a_mn, const voi
   p.D = D; p.ldd = ldd; p.out_f32 = out_f32;
   p.a_rows = kBlockM;
   p.a_mn = a_mn ? 1 : 0; p.b_mn = b_mn ? 1 : 0;
-  // 2-CTA tiles for the backward GEMMs too (G4R_GEMM_T_2SM=0: 1-CTA kernel); MN-major boxes are 64 x 64 either way
-  static int t2 = -1;
-  if (t2 < 0) { const char* e = getenv("G4R_GEMM_T_2SM"); t2 = (e && e[0] == '0') ? 0 : 1; }
-  const bool two = t2 && N % 256 == 0 && use_2sm(N, p.num_m_tiles, 1, false);
+  // 2-CTA tiles for the backward GEMMs too; MN-major boxes are 64 x 64 either way
+  const bool two = N % 256 == 0 && use_2sm(N, p.num_m_tiles, 1);
   const int bn = two ? 256 : pick_block_n(N, p.num_m_tiles, 1);
   p.num_n_tiles = (N + bn - 1) / bn;
   CUtensorMap ta, tb;
@@ -928,9 +916,7 @@ extern "C" int g4r_conv3x3_dw_bf16(const void* dz_pad, const void* x_pad_origin,
     int rc = make_tmap(&tb, x_pad_origin, 4, dims, str, box);
     if (rc) return rc;
   }
-  static int t2 = -1;
-  if (t2 < 0) { const char* e = getenv("G4R_GEMM_T_2SM"); t2 = (e && e[0] == '0') ? 0 : 1; }
-  if (t2 && use_2sm(p.N, p.num_m_tiles, 1, false)) return launch_gemm_2sm<false>(ta, tb, p, (cudaStream_t)stream);
+  if (use_2sm(p.N, p.num_m_tiles, 1)) return launch_gemm_2sm<false>(ta, tb, p, (cudaStream_t)stream);
   return launch_gemm<256, false>(ta, tb, p, (cudaStream_t)stream);
 }
 #endif
@@ -949,7 +935,7 @@ static int gemm_impl(const void* A, long long lda, const void* B, long long ldb,
   if (act == ACT_SWIGLU) G4R_REQUIRE(N % 2 == 0 && !out_f32 && k_splits == 1 && !residual, "SwiGLU epilogue: even N, bf16 out, no split-K/residual");
   if (k_splits > 1) G4R_REQUIRE(out_f32 && act == ACT_NONE && !residual && !bias, "split-K writes fp32 partial slabs [k_splits][M][ldd]: out_f32, no bias/act/residual");
   // M <= 16 (decode step): HBM-bound weight-streaming kernel instead of a mostly empty 128-row tile
-  if (M <= 16 && !out_f32 && k_splits == 1 && !residual_f32 && !bias_round_bf16 && skinny_enabled()) {
+  if (M <= 16 && !out_f32 && k_splits == 1 && !residual_f32 && !bias_round_bf16) {
     const int rc = gemm_skinny_dispatch(A, lda, B, ldb, D, ldd, M, N, K, bias, bias_f32, residual, ldr, act, rope_cos,
                                         rope_sin, rope_cols, rope_L, rope_pos0, rope_pos_dev, stream);
     if (rc >= 0) return rc;
@@ -968,7 +954,7 @@ static int gemm_impl(const void* A, long long lda, const void* B, long long ldb,
   p.rope_cols = rope_cols; p.rope_L = rope_L; p.rope_pos0 = rope_pos0; p.rope_pos_dev = rope_pos_dev;
   p.act = act; p.out_f32 = out_f32; p.atomic = k_splits > 1;
   p.conv = 0; p.a_rows = kBlockM;
-  const bool two = use_2sm(N, p.num_m_tiles, k_splits, false);
+  const bool two = use_2sm(N, p.num_m_tiles, k_splits);
   const int bn = two ? 256 : pick_block_n(N, p.num_m_tiles, k_splits);
   p.num_n_tiles = (N + bn - 1) / bn;
   CUtensorMap ta, tb;
@@ -1037,13 +1023,9 @@ extern "C" int g4r_conv_nhwc_bf16(const void* X, const void* Wt, void* Y, int n_
   p.k_splits = 1;
   p.D = Y; p.ldd = Cout; p.bias = bias; p.bias_f32 = bias_f32; p.act = act;
   p.conv = 1;
-  {
-    static int nf = -1;
-    if (nf < 0) { const char* e = getenv("G4R_CONV_NFAST"); nf = e ? atoi(e) : 1; }
-    p.n_fast = nf;
-  }
+  p.n_fast = 1;
   p.gn_stats = gn_stats; p.gn_groups = gn_groups; p.gn_group_ch = gn_groups ? Cout / gn_groups : 0;
-  const bool two = use_2sm(Cout, p.num_m_tiles, 1, true);
+  const bool two = use_2sm(Cout, p.num_m_tiles, 1);
   const int bn = two ? 256 : pick_block_n(Cout, p.num_m_tiles, 1);
   p.num_n_tiles = (Cout + bn - 1) / bn;
   CUtensorMap ta, tb;

@@ -377,13 +377,10 @@ __device__ __forceinline__ PackedAxis pack_axis(const AxisEntry<float>& e, int m
   return a;
 }
 
-// NV = 16-byte channel vectors per thread (1 or 2): with 2, the per-bin table reads, address arithmetic
-// and weight products are amortised over twice the channels (the kernel is issue / L1 bound, not HBM bound).
-template <typename Tin, typename Tout, int G, bool AFFINE, int NV>
-__global__ void __launch_bounds__(kThreads, (NV == 1 && sizeof(Tin) == 4 && !AFFINE ? 5 : 3))
+template <typename Tin, typename Tout, int G, bool AFFINE>
+__global__ void __launch_bounds__(kThreads, (sizeof(Tin) == 4 && !AFFINE ? 5 : 3))
 roi_align_fwd_nhwc_mlvl(const __grid_constant__ MlvlParams p) {
-  constexpr int VEC = 16 / (int)sizeof(Tin);
-  constexpr int CH = VEC * NV;
+  constexpr int VEC = 16 / (int)sizeof(Tin);   // channels per thread: one 16-byte vector
   __shared__ PackedAxis ytab[kTab];
   __shared__ PackedAxis xtab[kTab];
 
@@ -401,7 +398,7 @@ roi_align_fwd_nhwc_mlvl(const __grid_constant__ MlvlParams p) {
   const int gh = G > 0 ? G : g.gh, gw = G > 0 ? G : g.gw;
   // tables always fit for G > 0 (launcher guarantees PH*G, PW*G <= kTab); adaptive grids that do
   // not fit are processed in chunks of kTab samples per axis.
-  const int lanes = C / CH;
+  const int lanes = C / VEC;
   const Tin* map = reinterpret_cast<const Tin*>(p.maps[lvl]) + (size_t)g.batch * H * W * C;
   Tout* out = reinterpret_cast<Tout*>(p.out) +
               (((size_t)lvl * p.K + k) * p.PH + ph0) * (size_t)PW * C;
@@ -416,18 +413,18 @@ roi_align_fwd_nhwc_mlvl(const __grid_constant__ MlvlParams p) {
     __syncthreads();
     // Per-bin body: `prow`, `pw`, `lane` select the bin and the channel slice.
     auto do_bin = [&](int prow, int pw, int lane, const PackedAxis* eyp, const char* const* rows) {
-      const int coff = lane * CH;
+      const int coff = lane * VEC;
       const char* mpb = reinterpret_cast<const char*>(map + coff);
-      float ga[CH], gb[CH];
+      float ga[VEC], gb[VEC];
       if constexpr (AFFINE) {
         const float* sa = p.gn_scale[lvl] + (size_t)g.batch * C + coff;
         const float* sb = p.gn_shift[lvl] + (size_t)g.batch * C + coff;
 #pragma unroll
-        for (int i = 0; i < CH; i++) { ga[i] = sa[i]; gb[i] = sb[i]; }
+        for (int i = 0; i < VEC; i++) { ga[i] = sa[i]; gb[i] = sb[i]; }
       }
-      f32x2 acc2[CH / 2];
+      f32x2 acc2[VEC / 2];
 #pragma unroll
-      for (int i = 0; i < CH / 2; i++) acc2[i] = 0ull;   // (+0.f, +0.f)
+      for (int i = 0; i < VEC / 2; i++) acc2[i] = 0ull;   // (+0.f, +0.f)
 #pragma unroll
       for (int iy = 0; iy < (G > 0 ? G : gh); iy++) {
         const PackedAxis ey = eyp ? eyp[iy] : ytab[prow * gh + iy];
@@ -440,24 +437,16 @@ roi_align_fwd_nhwc_mlvl(const __grid_constant__ MlvlParams p) {
           const PackedAxis ex = xtab[pw * gw + ix];
           {
             const float w1 = ey.h * ex.h, w2 = ey.h * ex.l, w3 = ey.l * ex.h, w4 = ey.l * ex.l;
-            float v1[CH], v2[CH], v3[CH], v4[CH];
-#pragma unroll
-            for (int n = 0; n < NV; n++) {
-              float t1[VEC], t2[VEC], t3[VEC], t4[VEC];
-              load16_global<Tin>(r_lo + (size_t)(unsigned)ex.off_lo * 16 + n * 16, t1);
-              load16_global<Tin>(r_lo + (size_t)(unsigned)ex.off_hi * 16 + n * 16, t2);
-              load16_global<Tin>(r_hi + (size_t)(unsigned)ex.off_lo * 16 + n * 16, t3);
-              load16_global<Tin>(r_hi + (size_t)(unsigned)ex.off_hi * 16 + n * 16, t4);
-#pragma unroll
-              for (int i = 0; i < VEC; i++) {
-                v1[n * VEC + i] = t1[i]; v2[n * VEC + i] = t2[i]; v3[n * VEC + i] = t3[i]; v4[n * VEC + i] = t4[i];
-              }
-            }
+            float v1[VEC], v2[VEC], v3[VEC], v4[VEC];
+            load16_global<Tin>(r_lo + (size_t)(unsigned)ex.off_lo * 16, v1);
+            load16_global<Tin>(r_lo + (size_t)(unsigned)ex.off_hi * 16, v2);
+            load16_global<Tin>(r_hi + (size_t)(unsigned)ex.off_lo * 16, v3);
+            load16_global<Tin>(r_hi + (size_t)(unsigned)ex.off_hi * 16, v4);
             if constexpr (AFFINE) {
               // fused GroupNorm affine + ReLU on every tap (this engine's own fusion, tolerance-tested):
               // one FFMA2 per channel pair and tap
 #pragma unroll
-              for (int i = 0; i < CH; i += 2) {
+              for (int i = 0; i < VEC; i += 2) {
                 const f32x2 GA = pack2(ga[i], ga[i + 1]), GB = pack2(gb[i], gb[i + 1]);
                 float a, b;
                 unpack2(fma2(pack2(v1[i], v1[i + 1]), GA, GB), a, b); v1[i] = fmaxf(a, 0.f); v1[i + 1] = fmaxf(b, 0.f);
@@ -468,7 +457,7 @@ roi_align_fwd_nhwc_mlvl(const __grid_constant__ MlvlParams p) {
             }
             const f32x2 W1 = pack2(w1, w1), W2 = pack2(w2, w2), W3 = pack2(w3, w3), W4 = pack2(w4, w4);
 #pragma unroll
-            for (int i = 0; i < CH; i += 2) {
+            for (int i = 0; i < VEC; i += 2) {
               f32x2 t = mul2(W1, pack2(v1[i], v1[i + 1]));
               t = add2_unfused(t, mul2(W2, pack2(v2[i], v2[i + 1])), one2);
               t = add2_unfused(t, mul2(W3, pack2(v3[i], v3[i + 1])), one2);
@@ -478,18 +467,12 @@ roi_align_fwd_nhwc_mlvl(const __grid_constant__ MlvlParams p) {
           }
         }
       }
-      float acc[CH];
+      float acc[VEC];
 #pragma unroll
-      for (int i = 0; i < CH; i += 2) unpack2(acc2[i / 2], acc[i], acc[i + 1]);
+      for (int i = 0; i < VEC; i += 2) unpack2(acc2[i / 2], acc[i], acc[i + 1]);
 #pragma unroll
-      for (int i = 0; i < CH; i++) acc[i] = quarter ? acc[i] * 0.25f : acc[i] / g.count;
-#pragma unroll
-      for (int n = 0; n < NV; n++) {
-        float o[VEC];
-#pragma unroll
-        for (int i = 0; i < VEC; i++) o[i] = acc[n * VEC + i];
-        store_vec<Tout, VEC>(out + ((size_t)prow * PW + pw) * C + coff + n * VEC, o);
-      }
+      for (int i = 0; i < VEC; i++) acc[i] = quarter ? acc[i] * 0.25f : acc[i] / g.count;
+      store_vec<Tout, VEC>(out + ((size_t)prow * PW + pw) * C + coff, acc);
     };
     if constexpr (G > 0) {
       if (blockDim.x % lanes == 0 || lanes % blockDim.x == 0) {
@@ -500,7 +483,7 @@ roi_align_fwd_nhwc_mlvl(const __grid_constant__ MlvlParams p) {
           for (int prow = 0; prow < nrows; prow++) {
             PackedAxis eyr[G];
             const char* rows[2 * G];
-            const char* mpb = reinterpret_cast<const char*>(map + lane * CH);
+            const char* mpb = reinterpret_cast<const char*>(map + lane * VEC);
 #pragma unroll
             for (int iy = 0; iy < G; iy++) {
               eyr[iy] = ytab[prow * G + iy];
@@ -747,147 +730,6 @@ roi_align_fwd_nhwc_mlvl_dedup(const __grid_constant__ MlvlParams p) {
   }
 }
 
-// ------------------------------------------------------------------------------------
-// "Row walk" forward for the fixed 2x2 sampling grid (the SPI module's RoIAlign(14, sampling_ratio=2),
-// gpt4roi/models/layers.py:205-212, and the 7x7 microbench).
-//
-// The table kernel above is bound by L1 wavefronts: every bin-thread issues 16 16-byte tap loads for one
-// 16-byte store, although on the coarse levels consecutive samples of a bin row fall into the same or the
-// adjacent map column.  Here a thread owns a channel slice and a whole bin ROW: for each of the two sample
-// rows it walks the 2*PW x-samples left to right keeping the current (lo, hi) column pair of both map rows
-// in registers -- a sample whose columns are already held costs no load, a sample one column further
-// shifts hi -> lo and loads one column.  Loads drop to (distinct columns) x 2 rows per sample row; the
-// arithmetic (weights, association, accumulation order iy-major / ix-minor) is unchanged, so the result
-// stays bit-identical to the table kernel and to the reference CPU kernel.
-// ------------------------------------------------------------------------------------
-template <typename Tin, typename Tout, bool AFFINE>
-__global__ void __launch_bounds__(kThreads, (sizeof(Tin) == 4 ? 3 : 2))
-roi_align_fwd_nhwc_mlvl_walk(const __grid_constant__ MlvlParams p) {
-  constexpr int VEC = 16 / (int)sizeof(Tin);   // channels per thread
-  constexpr int NB = VEC == 4 ? 7 : 4;         // bins per walk segment (accumulators live in registers)
-  constexpr int G = 2;
-  __shared__ PackedAxis ytab[kTab];
-  __shared__ PackedAxis xtab[kTab];
-
-  const int lvl = blockIdx.y;
-  const int rpc = p.rows_per_cta_lvl[lvl];
-  const int row_groups = (p.PH + rpc - 1) / rpc;
-  const int k = blockIdx.x / row_groups;
-  if (k >= p.K) return;
-  const int ph0 = (blockIdx.x % row_groups) * rpc;
-  const int nrows = min(rpc, p.PH - ph0);
-  const int H = p.H[lvl], W = p.W[lvl], C = p.C, PW = p.PW;
-  const float* r = p.rois + (size_t)k * 5;
-  const RoiGeom<float> g = roi_geom<float>(r[0], r[1], r[2], r[3], r[4], p.scale[lvl], p.PH, PW, G, p.aligned != 0, true);
-  const int lanes = C / VEC;
-  const Tin* map = reinterpret_cast<const Tin*>(p.maps[lvl]) + (size_t)g.batch * H * W * C;
-  Tout* out = reinterpret_cast<Tout*>(p.out) + (((size_t)lvl * p.K + k) * p.PH + ph0) * (size_t)PW * C;
-  const f32x2 one2 = pack2(p.one, p.one);
-
-  for (int i = threadIdx.x; i < nrows * G; i += blockDim.x)
-    ytab[i] = pack_axis(axis_entry<float>(g.start_h, g.bin_h, ph0 + i / G, i % G, G, H), W * C);
-  for (int i = threadIdx.x; i < PW * G; i += blockDim.x)
-    xtab[i] = pack_axis(axis_entry<float>(g.start_w, g.bin_w, i / G, i % G, G, W), C * (int)sizeof(Tin) / 16);
-  __syncthreads();
-
-  // thread -> (channel slice, row group); blockDim.x is a multiple of lanes or lanes a multiple of blockDim.x
-  const int ngrp = blockDim.x >= lanes ? blockDim.x / lanes : 1;
-  const int rgrp = blockDim.x >= lanes ? threadIdx.x / lanes : 0;
-  for (int lane = threadIdx.x % lanes; lane < lanes; lane += (blockDim.x >= lanes ? lanes : blockDim.x)) {
-    const int coff = lane * VEC;
-    const char* mpb = reinterpret_cast<const char*>(map + coff);
-    f32x2 ga2[VEC / 2], gb2[VEC / 2];
-    if constexpr (AFFINE) {
-      const float* sa = p.gn_scale[lvl] + (size_t)g.batch * C + coff;
-      const float* sb = p.gn_shift[lvl] + (size_t)g.batch * C + coff;
-#pragma unroll
-      for (int i = 0; i < VEC; i += 2) { ga2[i / 2] = pack2(sa[i], sa[i + 1]); gb2[i / 2] = pack2(sb[i], sb[i + 1]); }
-    }
-    // one map pixel (16 bytes of channels) -> VEC/2 packed pairs, GroupNorm affine + ReLU applied once
-    auto load_px = [&](const char* ptr, f32x2 (&dst)[VEC / 2]) {
-      float t[VEC];
-      load16_global<Tin>(ptr, t);
-#pragma unroll
-      for (int i = 0; i < VEC; i += 2) {
-        if constexpr (AFFINE) {
-          float a, b;
-          unpack2(fma2(pack2(t[i], t[i + 1]), ga2[i / 2], gb2[i / 2]), a, b);
-          dst[i / 2] = pack2(fmaxf(a, 0.f), fmaxf(b, 0.f));
-        } else {
-          dst[i / 2] = pack2(t[i], t[i + 1]);
-        }
-      }
-    };
-    for (int prow = rgrp; prow < nrows; prow += ngrp) {
-      for (int pw0 = 0; pw0 < PW; pw0 += NB) {
-        f32x2 acc2[NB][VEC / 2];
-#pragma unroll
-        for (int b = 0; b < NB; b++)
-#pragma unroll
-          for (int i = 0; i < VEC / 2; i++) acc2[b][i] = 0ull;
-#pragma unroll
-        for (int iy = 0; iy < G; iy++) {
-          const PackedAxis ey = ytab[prow * G + iy];
-          const char* r_lo = mpb + (size_t)(unsigned)ey.off_lo * sizeof(Tin);
-          const char* r_hi = mpb + (size_t)(unsigned)ey.off_hi * sizeof(Tin);
-          unsigned c_lo = 0xffffffffu, c_hi = 0xffffffffu;        // columns currently held
-          f32x2 a_lo[VEC / 2], a_hi[VEC / 2], b_lo[VEC / 2], b_hi[VEC / 2];  // a: map row lo, b: map row hi
-#pragma unroll
-          for (int i = 0; i < VEC / 2; i++) a_lo[i] = a_hi[i] = b_lo[i] = b_hi[i] = 0ull;
-#pragma unroll
-          for (int j = 0; j < NB * G; j++) {
-            const int pw = pw0 + j / G;
-            if (pw < PW) {   // block-uniform
-              const PackedAxis ex = xtab[pw * G + (j % G)];
-              const unsigned xl = (unsigned)ex.off_lo, xh = (unsigned)ex.off_hi;
-              if (xl != c_lo || xh != c_hi) {   // warp-uniform: all lanes of a warp share the RoI and the row
-                if (xl == c_hi) {
-#pragma unroll
-                  for (int i = 0; i < VEC / 2; i++) { a_lo[i] = a_hi[i]; b_lo[i] = b_hi[i]; }
-                } else {
-                  load_px(r_lo + (size_t)xl * 16, a_lo);
-                  load_px(r_hi + (size_t)xl * 16, b_lo);
-                }
-                if (xh == xl) {
-#pragma unroll
-                  for (int i = 0; i < VEC / 2; i++) { a_hi[i] = a_lo[i]; b_hi[i] = b_lo[i]; }
-                } else {
-                  load_px(r_lo + (size_t)xh * 16, a_hi);
-                  load_px(r_hi + (size_t)xh * 16, b_hi);
-                }
-                c_lo = xl;
-                c_hi = xh;
-              }
-              // reference association: val = ((w1*v1 + w2*v2) + w3*v3) + w4*v4;  acc += val
-              const float w1 = ey.h * ex.h, w2 = ey.h * ex.l, w3 = ey.l * ex.h, w4 = ey.l * ex.l;
-              const f32x2 W1 = pack2(w1, w1), W2 = pack2(w2, w2), W3 = pack2(w3, w3), W4 = pack2(w4, w4);
-#pragma unroll
-              for (int i = 0; i < VEC / 2; i++) {
-                f32x2 t = mul2(W1, a_lo[i]);
-                t = add2_unfused(t, mul2(W2, a_hi[i]), one2);
-                t = add2_unfused(t, mul2(W3, b_lo[i]), one2);
-                t = add2_unfused(t, mul2(W4, b_hi[i]), one2);
-                acc2[j / G][i] = add2_unfused(acc2[j / G][i], t, one2);
-              }
-            }
-          }
-        }
-#pragma unroll
-        for (int b = 0; b < NB; b++) {
-          if (pw0 + b < PW) {
-            float o[VEC];
-#pragma unroll
-            for (int i = 0; i < VEC; i += 2) unpack2(acc2[b][i / 2], o[i], o[i + 1]);
-#pragma unroll
-            for (int i = 0; i < VEC; i++) o[i] = o[i] * 0.25f;   // count = 4: x/4 == x*0.25f exactly
-            store_vec<Tout, VEC>(out + ((size_t)prow * PW + pw0 + b) * C + coff, o);
-          }
-        }
-      }
-    }
-  }
-}
-
 // NHWC multi-level backward: grad_output [Lv,K,PH,PW,C] (Tg) -> fp32 NHWC grad maps (atomics).
 template <typename Tg>
 __global__ void __launch_bounds__(kThreads)
@@ -1001,15 +843,15 @@ static int launch_fwd_mlvl(MlvlParams& p, bool affine, cudaStream_t st) {
   // Rows per CTA, per level.  Whole-RoI CTAs amortise the table build; but on the big (fine)
   // levels a whole image-level does not fit L2 with many RoIs in flight, so those levels use one
   // bin row per CTA: ~PH x more CTAs per image => fewer images in flight => taps hit L2.
+  constexpr int VEC = 16 / (int)sizeof(Tin);
+  const int lanes = p.C / VEC;   // threads per bin: one 16-byte channel vector each
   int max_groups = 1;
-  const char* env = getenv("G4R_ROI_ROWS");
   for (int l = 0; l < p.n_levels; l++) {
     const double map_mb = (double)p.H[l] * p.W[l] * p.C * sizeof(Tin) / 1e6;
     int rows = map_mb > 8.0 ? 1 : pick_rows_per_cta(p.K, p.n_levels, p.PH);
-    if (env && atoi(env) > 0) rows = atoi(env);
-    // the row-walk kernel gives each thread group (C/VEC lanes) its own bin row: keep every group busy
-    const int lanes_l = p.C / (16 / (int)sizeof(Tin));
-    if (lanes_l < kThreads && rows < kThreads / lanes_l) rows = kThreads / lanes_l;
+    // At least kThreads / lanes bin rows per CTA.  This clamp was written for a row-walk kernel that gave each group
+    // of `lanes` threads its own bin row; the tap-dedup kernel was measured (DESIGN.md section 3) on the grid it shapes.
+    if (lanes < kThreads && rows < kThreads / lanes) rows = kThreads / lanes;
     if (rows > p.PH) rows = p.PH;
     p.rows_per_cta_lvl[l] = rows;
     const int groups = (p.PH + rows - 1) / rows;
@@ -1017,57 +859,20 @@ static int launch_fwd_mlvl(MlvlParams& p, bool affine, cudaStream_t st) {
   }
   dim3 grid((unsigned)(p.K * max_groups), p.n_levels);
   const bool g2 = p.sampling_ratio == 2 && p.PH * 2 <= kTab && p.PW * 2 <= kTab;
-  constexpr int VEC = 16 / (int)sizeof(Tin);
-  static int nv_env = -1;
-  if (nv_env < 0) {
-    const char* e = getenv("G4R_ROI_NV");
-    nv_env = e ? atoi(e) : 0;
-  }
-  // 2 vectors per thread only for fp32 maps (8 channels/thread); 16-bit maps already carry 8 per vector
-  // measured on B200 (profiles/r1_roialign_microbench_v3.jsonl): 2 vectors/thread is 25 % SLOWER (fewer
-  // threads per bin => less latency hiding), so it stays opt-in (G4R_ROI_NV=2)
-  const bool nv2 = sizeof(Tin) == 4 && p.C % (2 * VEC) == 0 && p.C / (2 * VEC) >= 32 && nv_env == 2;
-  // The row-walk kernel (fewer L1 wavefronts, but on-demand loads at 3 CTAs/SM) measured 9.7 ms against the
-  // table kernel's 7.6 ms on the BASELINE microbench (profiles/r1_roialign_microbench_v5.jsonl); an in-bin
-  // tap-dedup variant of the table kernel measured 10.7 ms.  Both lose to plain occupancy, so the walk kernel
-  // is opt-in (G4R_ROI_WALK=1) and the dedup variant was dropped.
-  static int walk_env = -1;
-  if (walk_env < 0) {
-    const char* e = getenv("G4R_ROI_WALK");
-    walk_env = e ? atoi(e) : 0;
-  }
-  const int lanes = p.C / VEC;
-  static int dedup_env = -1;
-  if (dedup_env < 0) {
-    const char* e = getenv("G4R_ROI_DEDUP");
-    dedup_env = e ? atoi(e) : 1;
-  }
-  if (g2 && dedup_env == 1 && walk_env != 1 && !nv2 && (kThreads % lanes == 0 || lanes % kThreads == 0)) {
+  // 2x2 sampling grid: the tap-dedup kernel (12.1 ms vs 15.3 ms for the table kernel on the BASELINE microbench).
+  // It maps threads to a fixed channel slice, so `lanes` must divide kThreads or be a multiple of it.
+  if (g2 && (kThreads % lanes == 0 || lanes % kThreads == 0)) {
     if (affine) roi_align_fwd_nhwc_mlvl_dedup<Tin, Tout, true><<<grid, kThreads, 0, st>>>(p);
     else roi_align_fwd_nhwc_mlvl_dedup<Tin, Tout, false><<<grid, kThreads, 0, st>>>(p);
     G4R_LAUNCH_CHECK("roi_align_fwd_nhwc_mlvl_dedup");
     return G4R_OK;
   }
-  if (g2 && walk_env == 1 && !nv2 && (kThreads % lanes == 0 || lanes % kThreads == 0)) {
-    if (affine) roi_align_fwd_nhwc_mlvl_walk<Tin, Tout, true><<<grid, kThreads, 0, st>>>(p);
-    else roi_align_fwd_nhwc_mlvl_walk<Tin, Tout, false><<<grid, kThreads, 0, st>>>(p);
-    G4R_LAUNCH_CHECK("roi_align_fwd_nhwc_mlvl_walk");
-    return G4R_OK;
-  }
   if (g2) {
-    if constexpr (sizeof(Tin) == 4) {
-      if (nv2) {
-        if (affine) roi_align_fwd_nhwc_mlvl<Tin, Tout, 2, true, 2><<<grid, kThreads, 0, st>>>(p);
-        else roi_align_fwd_nhwc_mlvl<Tin, Tout, 2, false, 2><<<grid, kThreads, 0, st>>>(p);
-      }
-    }
-    if (!nv2) {
-      if (affine) roi_align_fwd_nhwc_mlvl<Tin, Tout, 2, true, 1><<<grid, kThreads, 0, st>>>(p);
-      else roi_align_fwd_nhwc_mlvl<Tin, Tout, 2, false, 1><<<grid, kThreads, 0, st>>>(p);
-    }
+    if (affine) roi_align_fwd_nhwc_mlvl<Tin, Tout, 2, true><<<grid, kThreads, 0, st>>>(p);
+    else roi_align_fwd_nhwc_mlvl<Tin, Tout, 2, false><<<grid, kThreads, 0, st>>>(p);
   } else {
-    if (affine) roi_align_fwd_nhwc_mlvl<Tin, Tout, 0, true, 1><<<grid, kThreads, 0, st>>>(p);
-    else roi_align_fwd_nhwc_mlvl<Tin, Tout, 0, false, 1><<<grid, kThreads, 0, st>>>(p);
+    if (affine) roi_align_fwd_nhwc_mlvl<Tin, Tout, 0, true><<<grid, kThreads, 0, st>>>(p);
+    else roi_align_fwd_nhwc_mlvl<Tin, Tout, 0, false><<<grid, kThreads, 0, st>>>(p);
   }
   G4R_LAUNCH_CHECK("roi_align_fwd_nhwc_mlvl");
   return G4R_OK;

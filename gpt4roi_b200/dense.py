@@ -190,13 +190,13 @@ def conv_nhwc(x, weight_khwc, bias=None, act=None, gn_stats=None, out=None, leve
     return out
 
 
-def decode_gemm(x, weight, norm_w=None, norm_eps=1e-6, act=None, residual=None, rope=None, kv=None):
-    """Decode-step GEMM (M = batch <= 16): out = [RoPE | SwiGLU | + residual](RMSNorm(x) @ weight.T), the norm, the
-    rotary embedding and the KV-cache append folded into one weight-streaming launch (g4r_decode_gemm_bf16).
+def decode_gemm(x, weight, act=None, residual=None, rope=None, kv=None):
+    """Decode-step GEMM (M = batch <= 16): out = [RoPE | SwiGLU | + residual](x @ weight.T), the rotary embedding
+    and the KV-cache append folded into one weight-streaming launch (g4r_decode_gemm_bf16).
     rope = (cos, sin, rope_cols, pos0, pos_dev); kv = (kcache [B,Lmax,HD], vcache) -- needs rope on the fused q|k|v weight."""
     M, K = x.shape
     N = weight.shape[0]
-    dev = _L.require_cuda_same_device([('x', x), ('weight', weight), ('norm_w', norm_w), ('residual', residual)])
+    dev = _L.require_cuda_same_device([('x', x), ('weight', weight), ('residual', residual)])
     a16 = _act16('decode_gemm', x, weight)
     n_out = N // 2 if act == 'swiglu' else N
     out = torch.empty((M, n_out), dtype=a16, device=dev)
@@ -213,7 +213,7 @@ def decode_gemm(x, weight, norm_w=None, norm_eps=1e-6, act=None, residual=None, 
         _ps = _prof_begin(dev)
         _L.check(getattr(_L.load(), _L.sym('g4r_decode_gemm_bf16', a16))(
             _L.ptr(x), x.stride(0), _L.ptr(weight), weight.stride(0), _L.ptr(out), out.stride(0), M, N, K,
-            _L.ptr(norm_w), float(norm_eps), ACT[act], _L.ptr(residual), residual.stride(0) if residual is not None else 0,
+            ACT[act], _L.ptr(residual), residual.stride(0) if residual is not None else 0,
             _L.ptr(cos), _L.ptr(sin), int(rope_cols), int(pos0), _L.ptr(pos_dev), _L.ptr(kc), _L.ptr(vc), int(lmax), int(hd),
             _L.stream_ptr(dev)))
         _prof_end(dev, _ps, 'gemm', 2.0 * M * N * K)

@@ -378,7 +378,9 @@ class PrefillEngine:
                                    stage_taps=stage_taps)
 
 
-_DECODE_FUSED = int(__import__('os').environ.get('G4R_DECODE_FUSED', '1'))
+# Decode steps at B <= 16 take the fused GEMMs of g4r_decode_gemm_bf16; the unfused sequence remains the path for the
+# other shapes and the reference the tests compare the fused step against (they switch this off).
+_FUSED_DECODE = True
 
 
 class KVCache:
@@ -420,20 +422,18 @@ def _decode_step_chain(self, token_ids, cache, pos_dev):
     scale = c.head_dim ** -0.5
     fused = c.head_dim == 128 and (2 * c.hidden) % 256 == 0
     # KV-cache append folded into the q|k|v GEMM's RoPE epilogue (7 launches per layer instead of 8).  Folding the two
-    # RMSNorms into the GEMMs as well (G4R_DECODE_FUSED=2: 5 launches) measured SLOWER on B200 -- 4.57 vs 3.58 ms/token:
-    # the per-fragment normalisation sits between the weight-streaming loads of a kernel that lives on memory-level
-    # parallelism (profiles/r2_decode_fusion.md) -- so it stays opt-in.  G4R_DECODE_FUSED=0: the round-1 sequence.
-    fuse_step = fused and B <= 16 and c.hidden % 256 == 0 and _DECODE_FUSED > 0
+    # RMSNorms into the GEMMs as well (5 launches) measured SLOWER on B200 -- 4.57 vs 3.58 ms/token: the per-fragment
+    # normalisation sits between the weight-streaming loads of a kernel that lives on memory-level parallelism
+    # (profiles/r2_decode_fusion.md).
+    fuse_step = fused and B <= 16 and c.hidden % 256 == 0 and _FUSED_DECODE
     for li, w in enumerate(self.layers):
         if fuse_step:
-            nrm = _DECODE_FUSED >= 2
-            h = x if nrm else kernels.rmsnorm(x, w['ln_in'], c.rms_eps)
-            qkv = dense.decode_gemm(h, w['wqkv'], norm_w=w['ln_in'] if nrm else None, norm_eps=c.rms_eps,
-                                    rope=(cos, sin, 2 * c.hidden, pos, pos_dev), kv=(cache.k[li], cache.v[li]))
+            h = kernels.rmsnorm(x, w['ln_in'], c.rms_eps)
+            qkv = dense.decode_gemm(h, w['wqkv'], rope=(cos, sin, 2 * c.hidden, pos, pos_dev), kv=(cache.k[li], cache.v[li]))
             a = kernels.decode_attention(qkv, cache.k[li], cache.v[li], B, c.n_heads, c.head_dim, kv_len, scale, pos_dev)
             x = dense.linear(a, w['wo'], residual=x)
-            h = x if nrm else kernels.rmsnorm(x, w['ln_post'], c.rms_eps)
-            f = dense.decode_gemm(h, w['wgu'], norm_w=w['ln_post'] if nrm else None, norm_eps=c.rms_eps, act='swiglu')
+            h = kernels.rmsnorm(x, w['ln_post'], c.rms_eps)
+            f = dense.decode_gemm(h, w['wgu'], act='swiglu')
             x = dense.linear(f, w['wdown'], residual=x)
             continue
         h = kernels.rmsnorm(x, w['ln_in'], c.rms_eps)

@@ -79,11 +79,9 @@ def rope_inplace(qkv, cos, sin, L, n_heads_qk, head_dim):
     return qkv
 
 
-ATTN_IMPL = __import__('os').environ.get('G4R_ATTN', 'tc')  # 'tc' = tcgen05 kernel, 'mma' = mma.sync kernel
-
-
-def attention(qkv, B, L, n_heads, head_dim, causal, scale, out=None, seqlens=None, impl=None):
-    """qkv: packed bf16 [B*L, 3*n_heads*head_dim] = (q | k | v); returns [B*L, n_heads*head_dim]."""
+def attention(qkv, B, L, n_heads, head_dim, causal, scale, out=None, seqlens=None, impl='tc'):
+    """qkv: packed bf16 [B*L, 3*n_heads*head_dim] = (q | k | v); returns [B*L, n_heads*head_dim].
+    impl: 'tc' the tcgen05 kernel; 'mma' the mma.sync kernel, kept as the tests' cross-check."""
     act = _bf16(qkv)
     hd = n_heads * head_dim
     if out is None:
@@ -93,7 +91,7 @@ def attention(qkv, B, L, n_heads, head_dim, causal, scale, out=None, seqlens=Non
     base = qkv.data_ptr()
     import ctypes
     q, k, v = (ctypes.c_void_p(base + i * hd * esz) for i in range(3))
-    fn = 'g4r_attention_tc_bf16' if (impl or ATTN_IMPL) == 'tc' else 'g4r_attention_bf16'
+    fn = {'tc': 'g4r_attention_tc_bf16', 'mma': 'g4r_attention_bf16'}[impl]
     _call(fn, qkv.device, q, k, v, _L.ptr(out), ld, L * ld, out.stride(0), L * out.stride(0),
           B, n_heads, L, head_dim, int(bool(causal)), float(scale), _L.ptr(seqlens), act=act)
     return out

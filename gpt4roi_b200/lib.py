@@ -44,7 +44,7 @@ SIGNATURES = {
     'g4r_gemm_bf16_ex': (_i, [_vp, _ll, _vp, _ll, _vp, _ll, _i, _i, _i, _vp, _i, _vp, _ll, _i, _i, _i, _i, _i, _vp]),
     'g4r_gemm_bf16_t': (_i, [_vp, _ll, _i, _vp, _ll, _i, _vp, _ll, _i, _i, _i, _i, _vp]),
     'g4r_gemm_qkv_rope_bf16': (_i, [_vp, _ll, _vp, _ll, _vp, _ll, _i, _i, _i, _vp, _vp, _i, _i, _i, _vp, _vp]),
-    'g4r_decode_gemm_bf16': (_i, [_vp, _ll, _vp, _ll, _vp, _ll, _i, _i, _i, _vp, _f, _i, _vp, _ll, _vp, _vp, _i, _i, _vp, _vp, _vp,
+    'g4r_decode_gemm_bf16': (_i, [_vp, _ll, _vp, _ll, _vp, _ll, _i, _i, _i, _i, _vp, _ll, _vp, _vp, _i, _i, _vp, _vp, _vp,
                                   _i, _i, _vp]),
     'g4r_kv_append_bf16': (_i, [_vp, _ll, _vp, _vp, _i, _i, _i, _vp, _i, _i, _vp]),
     'g4r_decode_attention_bf16': (_i, [_vp, _ll, _vp, _vp, _vp, _ll, _i, _i, _i, _i, _vp, _i, _f, _vp]),
@@ -71,7 +71,6 @@ SIGNATURES = {
     'g4r_swiglu_fwd_bf16': (_i, [_vp, _ll, _vp, _ll, _ll, _i, _vp]),
     'g4r_swiglu_bwd_bf16': (_i, [_vp, _ll, _vp, _ll, _vp, _ll, _ll, _i, _vp]),
     'g4r_attention_tc_lse_bf16': (_i, [_vp] * 4 + [_ll] * 4 + [_i] * 5 + [_f, _vp, _vp]),
-    'g4r_attention_fwd_lse_bf16': (_i, [_vp] * 4 + [_ll] * 4 + [_i] * 5 + [_f, _vp, _vp]),
     'g4r_attention_bwd_bf16': (_i, [_vp] * 10 + [_ll] * 6 + [_i] * 5 + [_f, _vp]),
     'g4r_splice_backward': (_i, [_vp, _vp, _vp, _vp, _i, _i, _i, _i, _vp]),
     'g4r_embed_grad_rows': (_i, [_vp, _vp, _vp, _vp, _i, _vp, _i, _vp]),

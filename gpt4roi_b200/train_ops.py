@@ -198,9 +198,7 @@ def attention_fwd_lse(qkv, B, L, n_heads, head_dim, causal, scale):
     out = torch.empty((B * L, hid), dtype=BF16, device=qkv.device)
     lse = torch.empty((B, n_heads, L), dtype=torch.float32, device=qkv.device)
     ld = qkv.stride(0)
-    from .kernels import ATTN_IMPL
-    fn = 'g4r_attention_tc_lse_bf16' if ATTN_IMPL == 'tc' else 'g4r_attention_fwd_lse_bf16'   # G4R_ATTN=mma: mma.sync kernel
-    _call(fn, qkv.device, _L.ptr(qkv), _L.ptr(qkv[:, hid:]), _L.ptr(qkv[:, 2 * hid:]),
+    _call('g4r_attention_tc_lse_bf16', qkv.device, _L.ptr(qkv), _L.ptr(qkv[:, hid:]), _L.ptr(qkv[:, 2 * hid:]),
           _L.ptr(out), ld, L * ld, hid, L * hid, B, n_heads, L, head_dim, int(causal), float(scale), _L.ptr(lse))
     return out, lse
 

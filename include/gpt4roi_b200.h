@@ -48,8 +48,7 @@ int g4r_set_sm_reserve(int n_sms);
  * gpt4roi/app.py:293-300): while on != 0, the small-M GEMM, RMSNorm and single-query attention kernels are launched so
  * that each may start during its predecessor's tail, fetch its first WEIGHT block, and only then wait for the
  * predecessor.  Sound only for a launch sequence in which no kernel writes weights (the decode step); callers switch
- * it on around such a sequence and off again.  Returns the previous setting.  Process-wide; default off.
- * Env G4R_PDL=0 makes it a no-op, =2 releases dependents at kernel start instead of after the kernel's own wait. */
+ * it on around such a sequence and off again.  Returns the previous setting.  Process-wide; default off. */
 int g4r_set_pdl(int on);
 
 /* ---- RoIAlign: operator seam -------------------------------------------- */
@@ -225,14 +224,13 @@ int g4r_gemm_qkv_rope_bf16(const void* A, long long lda, const void* B, long lon
 /* ---- decode loop (KV cache) -------------------------------------------------- */
 /* Decode-step GEMM (M = batch <= 16 new tokens, one per sample; the LLaMA stack behind generate(), llava.py:263-283,
  * spi_llava.py:47-48), weight-streaming, with the neighbouring memory-bound steps folded in:
- *   out = [RoPE | SwiGLU | + residual]( RMSNorm_{norm_w, eps}(x) . W^T )
- * norm_w (optional, bf16 [K]): LlamaRMSNorm of the activation rows (modeling_llama.py:53-67, same rounding points as
- * g4r_rmsnorm_bf16) recomputed per CTA; rope_cos/sin (optional): rotate columns [0, rope_cols) at position pos0 / *pos_dev;
+ *   out = [RoPE | SwiGLU | + residual]( x . W^T )
+ * rope_cos/sin (optional): rotate columns [0, rope_cols) at position pos0 / *pos_dev;
  * kcache / vcache (optional, with RoPE on the fused q|k|v projection, N == 3 * cache_hd): the rotated key and the value
- * columns of sample m are also written to cache[m, pos, :] -- replaces g4r_rmsnorm_bf16 + g4r_gemm_qkv_rope_bf16 +
- * g4r_kv_append_bf16 (3 launches) and g4r_rmsnorm_bf16 + g4r_gemm_bf16_ex(swiglu) (2 launches) of the unfused step. */
+ * columns of sample m are also written to cache[m, pos, :] -- replaces g4r_gemm_qkv_rope_bf16 + g4r_kv_append_bf16
+ * (2 launches) of the unfused step. */
 int g4r_decode_gemm_bf16(const void* x, long long ldx, const void* W, long long ldw, void* out, long long ldo, int M,
-                         int N, int K, const void* norm_w, float norm_eps, int act, const void* residual, long long ldr,
+                         int N, int K, int act, const void* residual, long long ldr,
                          const void* rope_cos, const void* rope_sin, int rope_cols, int pos0, const int* pos_dev,
                          void* kcache, void* vcache, int cache_lmax, int cache_hd, void* stream);
 
@@ -378,15 +376,11 @@ int g4r_swiglu_fwd_bf16(const void* gu, long long ldg, void* f, long long ldf, l
 int g4r_swiglu_bwd_bf16(const void* gu, long long ldg, const void* df, long long ldf, void* dgu, long long ldd,
                         long long M, int F, void* stream);
 
-/* Causal attention for training: forward that also writes lse[B,H,L] (fp32 log-sum-exp of the scaled scores),
- * and the backward (autograd of transformers modeling_llama.py:199-222 eager attention): packed dQ|dK|dV rows
- * from q,k,v (after RoPE), the forward output `out`, `dout` and `lse`.  delta: fp32 scratch [B,H,L].
+/* Causal attention for training: forward on the tcgen05 / TMEM attention kernel that also writes lse[B,H,L] (fp32
+ * log-sum-exp of the scaled scores; q, k, v must be one packed [B*L, width] buffer, bs == L*ld), and the backward
+ * (autograd of transformers modeling_llama.py:199-222 eager attention): packed dQ|dK|dV rows from q,k,v (after
+ * RoPE), the forward output `out`, `dout` and `lse`.  delta: fp32 scratch [B,H,L].
  * q/k/v: row stride ld, batch stride bs (elements); out/dout: ldo, bso; dq/dk/dv: ldg, bsg.  No atomics. */
-int g4r_attention_fwd_lse_bf16(const void* q, const void* k, const void* v, void* out, long long ld,
-                               long long bs, long long ldo, long long bso, int B, int H, int L,
-                               int head_dim, int causal, float scale, float* lse, void* stream);
-/* Same contract on the tcgen05 / TMEM attention kernel (q, k, v must be one packed [B*L, width] buffer, bs == L*ld):
- * the training forward's default since round 2. */
 int g4r_attention_tc_lse_bf16(const void* q, const void* k, const void* v, void* out, long long ld, long long bs,
                               long long ldo, long long bso, int B, int H, int L, int head_dim, int causal, float scale,
                               float* lse, void* stream);
@@ -565,7 +559,7 @@ int g4r_affine_relu_nhwc_f16(const void* z, const float* scale, const float* shi
 int g4r_add_bias_pos_cast_f16(const float* acc, int splits, const void* bias, const float* pos, void* out,
                           int K, int D, void* stream);
 int g4r_decode_gemm_f16(const void* x, long long ldx, const void* W, long long ldw, void* out, long long ldo, int M,
-                         int N, int K, const void* norm_w, float norm_eps, int act, const void* residual, long long ldr,
+                         int N, int K, int act, const void* residual, long long ldr,
                          const void* rope_cos, const void* rope_sin, int rope_cols, int pos0, const int* pos_dev,
                          void* kcache, void* vcache, int cache_lmax, int cache_hd, void* stream);
 int g4r_kv_append_f16(const void* qkv, long long ld, void* kcache, void* vcache,

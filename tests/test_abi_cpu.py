@@ -127,6 +127,31 @@ def test_product_never_imports_oracle():
     assert not bad, 'product code references oracle/: %s' % bad
 
 
+def _env_switches_read(*dirs):
+    found = set()
+    for d in dirs:
+        for dp, _, fns in os.walk(os.path.join(ROOT, d)):
+            for fn in fns:
+                if fn.endswith(('.py', '.cu', '.cuh')):
+                    txt = open(os.path.join(dp, fn)).read()
+                    found |= set(re.findall(r'''getenv\(\s*"(G4R_[A-Z0-9_]+)"''', txt))
+                    found |= set(re.findall(r'''environ\.get\(\s*['"](G4R_[A-Z0-9_]+)['"]''', txt))
+    return found
+
+
+def test_every_environment_switch_is_documented():
+    """Every G4R_* variable the package reads is a row of the README's environment table, and every row is read
+    somewhere in the package or its tools: no undocumented knob, no documented knob that does nothing."""
+    readme = open(os.path.join(ROOT, 'README.md')).read()
+    table = readme.split('## Environment switches', 1)[1].split('\n## ', 1)[0]
+    rows = set(re.findall(r'^\|\s*`(G4R_[A-Z0-9_]+)`\s*\|', table, re.M))
+    assert rows
+    read = _env_switches_read('gpt4roi_b200')
+    assert read <= rows, 'read but not in the README table: %s' % sorted(read - rows)
+    unread = rows - _env_switches_read('gpt4roi_b200', 'tools')
+    assert not unread, 'in the README table but read nowhere: %s' % sorted(unread)
+
+
 def test_missing_library_fails_loudly(tmp_path, monkeypatch):
     from gpt4roi_b200 import lib
     monkeypatch.setattr(lib, '_lib', None)

@@ -1,6 +1,7 @@
 """Per-kernel timing of the decode step's kernels at 7B shapes, warm (back-to-back launches inside one
 CUDA graph, weights rotated over several copies so that every launch streams from HBM, not L2).
-usage: python tools/bench_skinny.py [batch]"""
+usage: python tools/bench_skinny.py [batch] [--pdl]"""
+import argparse
 import json
 import os
 import sys
@@ -38,8 +39,12 @@ def timed_graph(fn, n_iter=5):
 
 
 def main():
-    B = int(sys.argv[1]) if len(sys.argv) > 1 else 8
-    if os.environ.get('G4R_BENCH_PDL'):     # launch the chain the way the decode step does (programmatic dependent launch)
+    ap = argparse.ArgumentParser()
+    ap.add_argument('batch', nargs='?', type=int, default=8)
+    ap.add_argument('--pdl', action='store_true', help='launch the chain the way the decode step does (programmatic dependent launch)')
+    args = ap.parse_args()
+    B = args.batch
+    if args.pdl:
         from gpt4roi_b200 import lib
         lib.set_pdl(True)
     hid, ffn, H, D, V = 4096, 11008, 32, 128, 32006
@@ -66,12 +71,18 @@ def main():
 
     w = wset(3 * hid, hid)
     report('skinny qkv+rope 12288x4096', timed_graph(lambda: [dense.qkv_rope(x, wi, cos, sin, 1, 2 * hid, pos0=700) for wi in w]), R, 3 * hid * hid * 2)
-    del w
+    kc, vc = (torch.empty(B, Lmax, hid, device=DEV, dtype=BF) for _ in range(2))
+    report('decode_gemm qkv+rope+kv 12288x4096',
+           timed_graph(lambda: [dense.decode_gemm(x, wi, rope=(cos, sin, 2 * hid, 700, None), kv=(kc, vc)) for wi in w]), R,
+           3 * hid * hid * 2)
+    del w, kc, vc
     w = wset(hid, hid)
     report('skinny wo+residual 4096x4096', timed_graph(lambda: [dense.linear(x, wi, residual=res) for wi in w]), R, hid * hid * 2)
     del w
     w = wset(2 * ffn, hid)
     report('skinny gate/up swiglu 22016x4096', timed_graph(lambda: [dense.linear(x, wi, act='swiglu') for wi in w]), R, 2 * ffn * hid * 2)
+    report('decode_gemm gate/up swiglu 22016x4096', timed_graph(lambda: [dense.decode_gemm(x, wi, act='swiglu') for wi in w]), R,
+           2 * ffn * hid * 2)
     del w
     w = wset(hid, ffn)
     report('skinny down+residual 4096x11008', timed_graph(lambda: [dense.linear(xf, wi, residual=res) for wi in w]), R, ffn * hid * 2)
